@@ -191,3 +191,15 @@ def test_bench_helpers_without_a_gpu():
     assert max(rks) == 64 and max(Rk) == 4 and len(rks) == bench.D5 + 1 == 31
     m = bench.cfg5_flop_model()
     assert 1.3e10 < m["total"] < 1.5e10                 # SURVEY.md section 8(d)-5: ~13-14 GFLOP per vector
+    # --dump-outputs: each sampled vector is found exactly once over the ranks, worker threads and chunks, and the sample stays
+    # under 64 MB as float64 (rounded ranks <= 64, 16 bytes per complex entry)
+    for world, chunk, nw in ((1, 296, 3), (8, 100, 2), (3, 7, 4)):
+        found = []
+        for r in range(world):
+            first, nvec = t.shard_batch(bench.TOTAL5, r, world)
+            ids, plan = bench.dump_plan(first, nvec, chunk, nw)
+            found += [g for wi, pos in plan.items() for j, cols in pos.items() for b, g in cols
+                      if first + (j * nw + wi) * chunk + b == g and b < chunk]
+        assert sorted(found) == list(ids) and len(set(ids)) == bench.DUMP_SAMPLE
+    per_vector = sum(2 * min(rks[k], 64) * min(rks[k + 1], 64) * 16 for k in range(bench.D5))
+    assert bench.DUMP_SAMPLE * per_vector < 64e6
