@@ -63,12 +63,10 @@ void* ttn_stream(void);                   /* cudaStream_t the library launches o
 /* per-kernel-family CUDA-event timing on the library stream (bench.py's roofline pass; adds two event records per launch).
  * families: 0 gemm, 1 copy/permute, 2 apply, 3 qr panel, 4 qr reflector apply, 5 jacobi, 6 reductions/axpy, 7 gather/norms */
 #define TTN_NFAMILIES 8
-/* run-time switches, also readable from the environment at ttn_init: "gram_compress" (1: Gram path of tt_compress! for
- * truncerr == 0, csrc/heig.cu), "gram_jacobi_min" (columns from which the Gram-block Jacobi serves large SVDs),
- * "use_cholqr", "use_cluster_jacobi", "gemm_bulk" (1: TMA-staged Float64 big tile when the operands allow it),
- * "gemm_real_tile" (5: Float64 128x64 tile at two CTAs per SM, default; 0: the 128x128 one-CTA tile; 1/2/4, 3: timing variants),
- * "gemm_compact" (1: ComplexF64 64x64 two-stage tile at two CTAs per SM, default; 0: 64x128 / 64x64 four-stage tiles),
- * "gemm_thin" (1: streaming kernel for right-multiplications with N, K <= 32), "reset_flops"; read-only counters through
+/* run-time switches between two live paths on the same input (for tests that compare them): "gram_compress" (1: Gram path
+ * of tt_compress! for truncerr == 0, csrc/heig.cu), "gram_jacobi_min" (columns from which the Gram-block Jacobi serves large
+ * SVDs), "gemm_bulk" (1: TMA-staged Float64 big tile when the operands allow it), "gemm_thin" (1: streaming kernel for
+ * right-multiplications with N, K <= 32); "reset_flops" clears the flop counters; read-only counters through
  * ttn_get_option: "gemm_flops", "heig_flops", "gram_calls", "gram_fallbacks", "gram_last_flags".  Per host thread, like the context. */
 int ttn_set_option(const char* key, double value);
 int ttn_get_option(const char* key, double* value);

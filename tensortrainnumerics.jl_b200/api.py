@@ -74,7 +74,7 @@ def copy_synchronize() -> None:
 
 
 def set_option(key: str, value) -> None:
-    """run-time switch of the library (`ttn_set_option`): gram_compress, gram_jacobi_min, use_cholqr, use_cluster_jacobi"""
+    """run-time switch of the library (`ttn_set_option`): gram_compress, gram_jacobi_min, gemm_bulk, gemm_thin, reset_flops"""
     check(_lib.lib().ttn_set_option(key.encode(), float(value)))
 
 

@@ -50,13 +50,6 @@ int ttn_init(int device) {
     TTN_CUDA(cudaDeviceGetDefaultMemPool(&pool, device));
     uint64_t thr = UINT64_MAX;
     TTN_CUDA(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &thr));
-    c.use_cluster_jacobi = getenv("TTN_NO_CLUSTER_JACOBI") == nullptr;
-    c.use_cholqr = getenv("TTN_NO_CHOLQR") == nullptr;
-    c.gram_compress = !(getenv("TTN_GRAM_COMPRESS") && atoi(getenv("TTN_GRAM_COMPRESS")) == 0);
-    c.gemm_bulk = !(getenv("TTN_GEMM_BULK") && atoi(getenv("TTN_GEMM_BULK")) == 0);
-    c.gemm_compact = getenv("TTN_GEMM_COMPACT") ? atoi(getenv("TTN_GEMM_COMPACT")) : 1;
-    c.gemm_real_tile = getenv("TTN_GEMM_REAL_TILE") ? atoi(getenv("TTN_GEMM_REAL_TILE")) : 5;
-    if (const char* e = getenv("TTN_GRAM_JACOBI")) c.gram_jacobi_min = (atoi(e) != 0) ? 128 : (1 << 30);
     c.inited = true;
   }
   API_END
@@ -78,7 +71,7 @@ int ttn_shutdown(void) {
   API_END
 }
 
-// run-time switches (the environment variables of DESIGN.md section 3, settable after ttn_init: A/B timing and tests)
+// run-time switches that select between two live paths on the same input, so that tests can compare them; flop counters
 int ttn_set_option(const char* key, double value) {
   API_BEGIN
   need_init();
@@ -87,12 +80,8 @@ int ttn_set_option(const char* key, double value) {
   Context& c = ctx();
   if (k == "gram_compress") c.gram_compress = value != 0.0;
   else if (k == "gemm_bulk") c.gemm_bulk = value != 0.0;
-  else if (k == "gemm_compact") c.gemm_compact = (int)value;
-  else if (k == "gemm_real_tile") c.gemm_real_tile = (int)value;
   else if (k == "gemm_thin") c.gemm_thin = value != 0.0;
   else if (k == "gram_jacobi_min") c.gram_jacobi_min = (int)value;
-  else if (k == "use_cholqr") c.use_cholqr = value != 0.0;
-  else if (k == "use_cluster_jacobi") c.use_cluster_jacobi = value != 0.0;
   else if (k == "reset_flops") { c.flops_gemm = 0.0; c.flops_heig = 0.0; }
   else throw Error(TTN_EARG, "ttn_set_option: unknown key " + k);
   API_END
@@ -105,12 +94,8 @@ int ttn_get_option(const char* key, double* value) {
   const Context& c = ctx();
   if (k == "gram_compress") *value = c.gram_compress;
   else if (k == "gemm_bulk") *value = c.gemm_bulk;
-  else if (k == "gemm_compact") *value = c.gemm_compact;
-  else if (k == "gemm_real_tile") *value = c.gemm_real_tile;
   else if (k == "gemm_thin") *value = c.gemm_thin;
   else if (k == "gram_jacobi_min") *value = c.gram_jacobi_min;
-  else if (k == "use_cholqr") *value = c.use_cholqr;
-  else if (k == "use_cluster_jacobi") *value = c.use_cluster_jacobi;
   else if (k == "gemm_flops") *value = c.flops_gemm;
   else if (k == "heig_flops") *value = c.flops_heig;
   else if (k == "gram_calls") *value = (double)c.gram_calls;

@@ -16,11 +16,6 @@
 
 namespace ttn {
 
-// TTN_DEBUG_SVD=1 prints one line per factorisation (read once)
-static inline bool debug_svd() {
-  static const bool on = getenv("TTN_DEBUG_SVD") != nullptr;
-  return on;
-}
 namespace {
 
 constexpr int CQ_T = 256;

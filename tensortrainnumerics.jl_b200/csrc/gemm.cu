@@ -333,7 +333,6 @@ void launch_cfg(const GemmArgs& g) {
     TTN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_dev = ctx().device;
   }
-  const int64_t nb = (int64_t)g.batch1 * g.batch2;
   // grid.z is limited to 65535: split the outer batch dimension if needed
   const int64_t max_b2 = std::max<int64_t>(1, 65535 / g.batch1);
   ttn_assert(g.batch1 <= 65535, 2, "gemm: inner batch dimension too large");
@@ -352,7 +351,6 @@ void launch_cfg(const GemmArgs& g) {
     TTN_CHECK_LAUNCH();
     ctx().launches++;
   }
-  (void)nb;
 }
 
 template <class T, int BM, int BN, int WM, int WN, int NS = NSTAGE>
@@ -443,55 +441,33 @@ bool try_thin(const GemmArgs& g) {
   return true;
 }
 
-template <class T> struct Tiles;
-template <> struct Tiles<double> {
-  static void big(const GemmArgs& g) { launch_major<double, 128, 128, 64, 32>(g); }
-  static void small(const GemmArgs& g) { launch_major<double, 64, 64, 32, 16>(g); }
-  static void compact(const GemmArgs& g) {
-    const int v = ctx().gemm_real_tile;
-    if (v == 1) launch_major<double, 128, 64, 32, 32, 3>(g);
-    else if (v == 2) launch_major<double, 128, 64, 32, 32, 2>(g);
-    else if (v == 4) launch_major<double, 128, 64, 32, 32, 4>(g);
-    else if (v == 5) { if (!try_bulk<double, 128, 64, 32, 32>(g)) launch_major<double, 128, 64, 32, 32, 3>(g); }
-    else launch_major<double, 64, 64, 32, 16, 2>(g);
-  }
-  static constexpr int BIGM = 128, BIGN = 128;
-};
-template <> struct Tiles<zc> {
-  static void big(const GemmArgs& g) { launch_major<zc, 64, 128, 32, 32>(g); }
-  static void small(const GemmArgs& g) { launch_major<zc, 64, 64, 32, 16>(g); }
-  // 64 x 64 tile, two pipeline stages: 68 KB of shared memory and 32 K registers per CTA, so that one such CTA fits on an SM next
-  // to a CTA of the (latency-bound, 132 KB) ComplexF64 tridiagonalisation kernel of another stream (ctx().gemm_compact)
-  static void compact(const GemmArgs& g) {
-    const int v = ctx().gemm_compact;
-    if (v == 2) launch_major<zc, 64, 64, 32, 16, 3>(g);
-    else if (v == 3) launch_major<zc, 64, 64, 32, 16, 4>(g);
-    else launch_major<zc, 64, 64, 32, 16, 2>(g);
-  }
-  static constexpr int BIGM = 64, BIGN = 128;
-};
-
 }  // namespace
 
 template <class T>
 void gemm(const GemmArgs& g) {
   if (g.M <= 0 || g.N <= 0 || g.batch1 <= 0 || g.batch2 <= 0) return;
   ProfScope prof_scope_(KF_GEMM);
-  ctx().flops_gemm += gemm_flops(g, is_cplx<T>::value);
-  const int64_t ctas_big = (int64_t)((g.M + Tiles<T>::BIGM - 1) / Tiles<T>::BIGM) *
-                           ((g.N + Tiles<T>::BIGN - 1) / Tiles<T>::BIGN) * g.batch1 * g.batch2;
-  const bool big = g.M >= (Tiles<T>::BIGM * 3) / 4 && g.N >= (Tiles<T>::BIGN * 3) / 4 &&
-                   ctas_big >= (int64_t)(ctx().sm_count * 3) / 4;
+  constexpr bool cplx = is_cplx<T>::value;
+  ctx().flops_gemm += gemm_flops(g, cplx);
+  // a "big" product fills 3/4 of a 128 x 128 (Float64) / 64 x 128 (ComplexF64) tile and, with such tiles, 3/4 of the SMs
+  constexpr int BIGM = cplx ? 64 : 128, BIGN = 128;
+  const int64_t ctas_big = (int64_t)((g.M + BIGM - 1) / BIGM) * ((g.N + BIGN - 1) / BIGN) * g.batch1 * g.batch2;
+  const bool big = g.M >= (BIGM * 3) / 4 && g.N >= (BIGN * 3) / 4 && ctas_big >= (int64_t)(ctx().sm_count * 3) / 4;
   if (ctx().gemm_thin && try_thin<T>(g)) return;
-  if (g.npeer == 0 && (is_cplx<T>::value ? ctx().gemm_compact != 0 : (ctx().gemm_real_tile != 0 && big))) {
-    Tiles<T>::compact(g);
-    return;
-  }
-  if (big) {
-    if (!is_cplx<T>::value && try_bulk<double, 128, 128, 64, 32>(g)) return;
-    Tiles<T>::big(g);
+  if (g.npeer != 0) {
+    // fused all-gather epilogue (two or more GPUs): four-stage tiles, one CTA per SM on the big ones
+    if (!big) launch_major<T, 64, 64, 32, 16>(g);
+    else if constexpr (cplx) launch_major<zc, 64, 128, 32, 32>(g);
+    else launch_major<double, 128, 128, 64, 32>(g);
+  } else if constexpr (cplx) {
+    // 64 x 64 tile, two pipeline stages: 68 KB of shared memory and 32 K registers per CTA, so that one such CTA fits on an SM next
+    // to a CTA of the (latency-bound, 132 KB) ComplexF64 tridiagonalisation kernel of another stream
+    launch_major<zc, 64, 64, 32, 16, 2>(g);
+  } else if (big) {
+    // 128 x 64 tile at two CTAs per SM: TMA-staged when the operands allow it, else three LDGSTS stages
+    if (!try_bulk<double, 128, 64, 32, 32>(g)) launch_major<double, 128, 64, 32, 32, 3>(g);
   } else {
-    Tiles<T>::small(g);
+    launch_major<double, 64, 64, 32, 16>(g);
   }
 }
 

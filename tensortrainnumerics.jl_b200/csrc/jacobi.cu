@@ -20,11 +20,6 @@ namespace ttn {
 namespace {
 
 constexpr int JAC_MAX_SWEEPS = 40;
-// Optional noise floor (Context::jacobi_noise_floor, off by default): a column whose squared norm is below
-// JAC_FLOOR2 * ||X||_F^2 (norm below 16 eps ||X||_F) is left alone instead of being orthogonalised to full relative
-// precision.  Off by default because the null-space vectors then come back non-orthogonal; rank-deficient bonds of
-// tt_compress! are handled by the factored split in tt.cu instead.
-constexpr double JAC_FLOOR2 = 3.2e-30;
 
 __device__ __forceinline__ double wsumd(double v) {
 #pragma unroll
@@ -68,7 +63,6 @@ template <class T, int GL, int RPL, bool FULLM>
 __global__ void __launch_bounds__(JAC_T) jacobi_kernel(T* __restrict__ X, int m, int64_t ldx, int64_t bX,
                                                        const int* __restrict__ grpA, const int* __restrict__ grpB, int bsz,
                                                        int n, int mode, int full, int sweeps, double tol,
-                                                       const double* __restrict__ d_frob2, double floor_k,
                                                        unsigned int* __restrict__ d_rotated, int* __restrict__ d_sweeps) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_rot;
@@ -78,7 +72,6 @@ __global__ void __launch_bounds__(JAC_T) jacobi_kernel(T* __restrict__ X, int m,
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
   const int grp = tid / GL, ngrp = blockDim.x / GL, gl = tid % GL;
   const double tol2 = tol * tol;
-  const double floor2 = floor_k * d_frob2[blockIdx.y];   // columns below sqrt(floor_k) ||X||_F are treated as numerically zero
   const int pitch = m + PADC;
 
   const int a0 = grpA[blockIdx.x] * bsz;
@@ -165,7 +158,7 @@ __global__ void __launch_bounds__(JAC_T) jacobi_kernel(T* __restrict__ X, int m,
           if (act) {
             const double b = nrm2[q];
             const double c2 = cr * cr + ci * ci;
-            if (c2 > tol2 * an * b && an > floor2 && b > floor2) {   // false for zero / noise-level columns and NaNs
+            if (c2 > tol2 * an * b && an > 0.0 && b > 0.0) {   // false for zero columns and NaNs
               double cs, sn, absc, phr, phi;
               if (is_cplx<T>::value) {
                 const double inv = rsqrt(c2);
@@ -246,14 +239,12 @@ __global__ void __launch_bounds__(JAC_T) jacobi_kernel(T* __restrict__ X, int m,
 template <class T, int RPLA>
 __global__ void __launch_bounds__(JAC_T) jacobi_cross_kernel(T* __restrict__ X, int m, int64_t ldx, int64_t bX,
                                                              const int* __restrict__ grpA, const int* __restrict__ grpB,
-                                                             int bsz, int n, double tol, const double* __restrict__ d_frob2, double floor_k,
-                                                             unsigned int* __restrict__ d_rotated) {
+                                                             int bsz, int n, double tol, unsigned int* __restrict__ d_rotated) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   T* Xb = X + blockIdx.y * bX;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int NW = JAC_T / 32;
   const double tol2 = tol * tol;
-  const double floor2 = floor_k * d_frob2[blockIdx.y];
   const int a0 = grpA[blockIdx.x] * bsz, na = min(bsz, n - a0);
   const int b0 = grpB[blockIdx.x] * bsz, nb = min(bsz, n - b0);
   const int pitch = m + (is_cplx<T>::value ? 0 : 4);
@@ -304,7 +295,7 @@ __global__ void __launch_bounds__(JAC_T) jacobi_cross_kernel(T* __restrict__ X, 
       if (act) {
         const double b = nrmB[bq];
         const double c2 = cr * cr + ci * ci;
-        if (c2 > tol2 * an * b && an > floor2 && b > floor2) {
+        if (c2 > tol2 * an * b && an > 0.0 && b > 0.0) {
           double cs, sn, absc, phr, phi;
           if (is_cplx<T>::value) {
             const double inv = rsqrt(c2);
@@ -352,24 +343,6 @@ __global__ void __launch_bounds__(JAC_T) jacobi_cross_kernel(T* __restrict__ X, 
 template <class T> struct JacCfg;
 template <> struct JacCfg<double> { static constexpr int GL = 4, RPL = 32, GLG = 8; };
 template <> struct JacCfg<zc> { static constexpr int GL = 8, RPL = 16, GLG = 8; };
-
-template <class T>
-__global__ void frob2_kernel(const T* __restrict__ X, int m, int n, int64_t ldx, int64_t bX, double* __restrict__ out) {
-  const T* Xb = X + blockIdx.y * bX;
-  double a = 0.0;
-  const int64_t total = (int64_t)m * n;
-  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < total; idx += (int64_t)gridDim.x * blockDim.x)
-    a += t_abs2(Xb[(idx / m) * ldx + idx % m]);
-  a = wsumd(a);
-  __shared__ double part[8];
-  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = a;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += part[w];
-    atomicAdd(out + blockIdx.y, s);
-  }
-}
 
 template <class T>
 __global__ void colnorm_kernel(const T* __restrict__ X, int m, int n, int64_t ldx, int64_t bX, double* __restrict__ norms,
@@ -425,19 +398,8 @@ int jacobi_orth(T* X, int m, int n, int64_t ldx, double* norms, int batch, int64
   const int threads = JAC_T;
   int sweeps_used = 0;
   ttn_assert(2 * col_bytes <= budget, 2, "jacobi: a column pair does not fit in shared memory");
-  DevBuf dsw_cl(sizeof(int) * batch), frob2(sizeof(double) * batch);
-  TTN_CUDA(cudaMemsetAsync(frob2.p, 0, frob2.bytes, ctx().stream));
-  for (int b0 = 0; b0 < batch; b0 += 65535) {
-    const int nb = std::min(65535, batch - b0);
-    const int blocks = (int)std::min<int64_t>(((int64_t)m * n + 2047) / 2048, 64);
-    ProfScope prof_scope_(KF_GATHER);
-    frob2_kernel<T><<<dim3(blocks, nb), 256, 0, ctx().stream>>>(X + (int64_t)b0 * bX, m, n, ldx, bX, frob2.as<double>() + b0);
-    TTN_CHECK_LAUNCH();
-    ctx().launches++;
-  }
-  const double* fr = frob2.as<double>();
-  const double fk = ctx().jacobi_noise_floor ? JAC_FLOOR2 : 0.0;
-  if (ctx().use_cluster_jacobi && jacobi_cluster<T>(X, m, n, ldx, batch, bX, tol, fr, fk, dsw_cl.as<int>())) {
+  DevBuf dsw_cl(sizeof(int) * batch);
+  if (jacobi_cluster<T>(X, m, n, ldx, batch, bX, tol, dsw_cl.as<int>())) {
     int hsw = 0;
     read_back(&hsw, dsw_cl.p, sizeof(int));
     sweeps_used = hsw;
@@ -451,7 +413,7 @@ int jacobi_orth(T* X, int m, int n, int64_t ldx, double* norms, int batch, int64
       dim3 grid(1, nb);
       ProfScope prof_scope_(KF_JACOBI);
       kern<<<grid, threads, (size_t)n * col_bytes, ctx().stream>>>(X + (int64_t)b0 * bX, m, ldx, bX, grp.as<int>(),
-                                                                 grp.as<int>() + 1, n, n, 0, 1, 0, tol, fr + b0, fk, nullptr,
+                                                                 grp.as<int>() + 1, n, n, 0, 1, 0, tol, nullptr,
                                                                  dsw.as<int>() + b0);
       TTN_CHECK_LAUNCH();
       ctx().launches++;
@@ -462,7 +424,7 @@ int jacobi_orth(T* X, int m, int n, int64_t ldx, double* norms, int batch, int64
   } else if (n >= 128 && m >= 64 && std::min(m, n) >= ctx().gram_jacobi_min) {
     // large matrices: Gram-block Jacobi, O(m n^2) work on the FP64 tensor pipe (jacobi_gram.cu)
     for (int b = 0; b < batch; ++b) {
-      const int sw = jacobi_gram<T>(X + (int64_t)b * bX, m, n, ldx, tol, fr + b, fk, JAC_MAX_SWEEPS);
+      const int sw = jacobi_gram<T>(X + (int64_t)b * bX, m, n, ldx, tol, JAC_MAX_SWEEPS);
       ttn_assert(sw >= 0, 7, "jacobi_gram: shape not served");
       if (b == 0) sweeps_used = sw;
     }
@@ -519,13 +481,13 @@ int jacobi_orth(T* X, int m, int n, int64_t ldx, double* norms, int batch, int64
         if (st == 0 || !fast) {
           const size_t smem = (size_t)(st == 0 ? 1 : 2) * bsz * col_bytes;
           gen<<<grid, threads, smem, ctx().stream>>>(X, m, ldx, bX, gA.as<int>() + off[st], gB.as<int>() + off[st], bsz, n,
-                                                    st == 0 ? 0 : 1, 0, 1, tol, fr, fk, dmax.as<unsigned int>(), nullptr);
+                                                    st == 0 ? 0 : 1, 0, 1, tol, dmax.as<unsigned int>(), nullptr);
         } else if (small_rows) {
           jacobi_cross_kernel<T, RPLA_S><<<grid, threads, (size_t)bsz * col_bytes, ctx().stream>>>(
-              X, m, ldx, bX, gA.as<int>() + off[st], gB.as<int>() + off[st], bsz, n, tol, fr, fk, dmax.as<unsigned int>());
+              X, m, ldx, bX, gA.as<int>() + off[st], gB.as<int>() + off[st], bsz, n, tol, dmax.as<unsigned int>());
         } else {
           jacobi_cross_kernel<T, RPLA_L><<<grid, threads, (size_t)bsz * col_bytes, ctx().stream>>>(
-              X, m, ldx, bX, gA.as<int>() + off[st], gB.as<int>() + off[st], bsz, n, tol, fr, fk, dmax.as<unsigned int>());
+              X, m, ldx, bX, gA.as<int>() + off[st], gB.as<int>() + off[st], bsz, n, tol, dmax.as<unsigned int>());
         }
         TTN_CHECK_LAUNCH();
         ctx().launches++;

@@ -42,7 +42,7 @@ __device__ __forceinline__ void next_slot(int c, bool top, int& dc, bool& dtop) 
 // One plane rotation of the column pair held in registers (rp, rq: RPL rows per lane of a GL-lane group) with maintained
 // squared norms an, bn.  Returns 0 (skipped), 1 (rotated, |x_p^H x_q|^2 <= 1e-18 a b and sin^2 <= 1e-10) or 2 (rotated).
 template <class T, int GL, int RPL>
-__device__ __forceinline__ int rotate_pair(T (&rp)[RPL], T (&rq)[RPL], double& an, double& bn, double tol2, double floor2) {
+__device__ __forceinline__ int rotate_pair(T (&rp)[RPL], T (&rq)[RPL], double& an, double& bn, double tol2) {
   T c2v[2] = {t_zero<T>(), t_zero<T>()};
 #pragma unroll
   for (int k = 0; k < RPL; ++k) t_fma(c2v[k & 1], t_conj(rp[k]), rq[k]);
@@ -55,7 +55,7 @@ __device__ __forceinline__ int rotate_pair(T (&rp)[RPL], T (&rq)[RPL], double& a
   }
   const double cc = cr * cr + ci * ci;
   const double ab = an * bn;
-  if (!(cc > tol2 * ab) || !(an > floor2) || !(bn > floor2)) return 0;   // group-uniform; zero / noise-level columns, NaNs
+  if (!(cc > tol2 * ab) || !(an > 0.0) || !(bn > 0.0)) return 0;   // group-uniform; zero columns, NaNs
   double absc, phr, phi;
   if (is_cplx<T>::value) {
     const double inv = rsqrt(cc);
@@ -107,8 +107,7 @@ __device__ __forceinline__ void send_column(cg::cluster_group& cluster, T* cols,
 // of a block step from the remote stores — half the shared memory, used to pack a batch of matrices onto the SMs.
 template <class T, int CL, int GL, int RPL, bool DB>
 __global__ void __launch_bounds__(512) jacobi_cluster_kernel(T* __restrict__ X, int m, int n, int64_t ldx, int64_t bX, int W,
-                                                              double tol, const double* __restrict__ d_frob2, double floor_k,
-                                                              int* __restrict__ d_sweeps) {
+                                                              double tol, int* __restrict__ d_sweeps) {
   cg::cluster_group cluster = cg::this_cluster();
   const int crank = (int)cluster.block_rank();
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -123,7 +122,6 @@ __global__ void __launch_bounds__(512) jacobi_cluster_kernel(T* __restrict__ X, 
   const int tid = threadIdx.x;
   const int grp = tid / GL, gl = tid % GL;               // grp < W
   const double tol2 = tol * tol;
-  const double floor2 = floor_k * d_frob2[blockIdx.x / CL];   // optional noise floor (jacobi.cu JAC_FLOOR2), 0 = off
   T* Xb = X + (int64_t)(blockIdx.x / CL) * bX;           // grid.x = CL * batch
   const int col0 = crank * ncl;
 
@@ -169,7 +167,7 @@ __global__ void __launch_bounds__(512) jacobi_cluster_kernel(T* __restrict__ X, 
 #pragma unroll
           for (int k = 0; k < RPL; ++k) { rp[k] = xp[k * GL]; rq[k] = xq[k * GL]; }
           double an = nb[p], bn = nb[q];
-          lvl = max(lvl, rotate_pair<T, GL, RPL>(rp, rq, an, bn, tol2, floor2));
+          lvl = max(lvl, rotate_pair<T, GL, RPL>(rp, rq, an, bn, tol2));
           if (r + 1 < M1) {
 #pragma unroll
             for (int k = 0; k < RPL; ++k) { xp[k * GL] = rp[k]; xq[k * GL] = rq[k]; }
@@ -198,7 +196,7 @@ __global__ void __launch_bounds__(512) jacobi_cluster_kernel(T* __restrict__ X, 
 #pragma unroll
           for (int k = 0; k < RPL; ++k) rq[k] = xq[k * GL];
           double bn = nb[q];
-          lvl = max(lvl, rotate_pair<T, GL, RPL>(rp, rq, an, bn, tol2, floor2));
+          lvl = max(lvl, rotate_pair<T, GL, RPL>(rp, rq, an, bn, tol2));
           if (r + 1 < W) {
 #pragma unroll
             for (int k = 0; k < RPL; ++k) xq[k * GL] = rq[k];
@@ -243,7 +241,7 @@ __global__ void __launch_bounds__(512) jacobi_cluster_kernel(T* __restrict__ X, 
 }
 
 template <class T, int CL, int GL, int RPL, bool DB>
-bool launch_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, const double* frob2, double fk, int* d_sweeps) {
+bool launch_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, int* d_sweeps) {
   const int W = (n + 2 * CL - 1) / (2 * CL);
   const int threads = W * GL;
   if (threads > 512 || threads < 32 || (threads & 31)) return false;
@@ -270,7 +268,7 @@ bool launch_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, doub
     cfg.attrs = at;
     cfg.numAttrs = 1;
     ProfScope prof_scope_(KF_JACOBI);
-    TTN_CUDA(cudaLaunchKernelEx(&cfg, kern, X + (int64_t)b0 * bX, m, n, ldx, bX, W, tol, frob2 + b0, fk, d_sweeps + b0));
+    TTN_CUDA(cudaLaunchKernelEx(&cfg, kern, X + (int64_t)b0 * bX, m, n, ldx, bX, W, tol, d_sweeps + b0));
     ctx().launches++;
   }
   return true;
@@ -283,30 +281,30 @@ bool launch_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, doub
 //   large batches : the smallest cluster whose shared memory holds the matrix (2 or 4 CTAs, single buffer), so that
 //                   sm_count/CL matrices are in flight at once (cfg5: ComplexF64 128 x 128 does not fit in one SM).
 template <class T>
-bool jacobi_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, const double* frob2, double fk, int* d_sweeps) {
+bool jacobi_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, int* d_sweeps) {
   if (n < 32) return false;                       // tiny problems: one SM is enough
   const bool few = batch * 8 <= ctx().sm_count;
   if (few) {
-    if (m <= 128) return launch_cluster<T, 8, 32, 4, true>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps);
-    if (m <= 256) return launch_cluster<T, 8, 32, 8, true>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps);
+    if (m <= 128) return launch_cluster<T, 8, 32, 4, true>(X, m, n, ldx, batch, bX, tol, d_sweeps);
+    if (m <= 256) return launch_cluster<T, 8, 32, 8, true>(X, m, n, ldx, batch, bX, tol, d_sweeps);
     return false;
   }
   const size_t one_sm = (sizeof(T) * (size_t)(m + 4) + 8) * n;   // footprint of the single-SM kernel (jacobi.cu)
   if (one_sm <= 216 * 1024) return false;         // fits in one SM: one matrix per SM is the throughput-optimal layout
   if (m <= 128) {
     // 4 CTAs x 64 KB (two clusters' CTAs co-resident per SM) measured 5 % faster than 2 CTAs x 128 KB on cfg5
-    if (n <= 256 && launch_cluster<T, 4, 16, 8, false>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps)) return true;
-    if (n <= 128 && launch_cluster<T, 2, 16, 8, false>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps)) return true;
-    return launch_cluster<T, 8, 32, 4, false>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps);
+    if (n <= 256 && launch_cluster<T, 4, 16, 8, false>(X, m, n, ldx, batch, bX, tol, d_sweeps)) return true;
+    if (n <= 128 && launch_cluster<T, 2, 16, 8, false>(X, m, n, ldx, batch, bX, tol, d_sweeps)) return true;
+    return launch_cluster<T, 8, 32, 4, false>(X, m, n, ldx, batch, bX, tol, d_sweeps);
   }
   if (m <= 256) {
-    if (launch_cluster<T, 4, 32, 8, false>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps)) return true;
-    return launch_cluster<T, 8, 32, 8, false>(X, m, n, ldx, batch, bX, tol, frob2, fk, d_sweeps);
+    if (launch_cluster<T, 4, 32, 8, false>(X, m, n, ldx, batch, bX, tol, d_sweeps)) return true;
+    return launch_cluster<T, 8, 32, 8, false>(X, m, n, ldx, batch, bX, tol, d_sweeps);
   }
   return false;
 }
 
-template bool jacobi_cluster<double>(double*, int, int, int64_t, int, int64_t, double, const double*, double, int*);
-template bool jacobi_cluster<zc>(zc*, int, int, int64_t, int, int64_t, double, const double*, double, int*);
+template bool jacobi_cluster<double>(double*, int, int, int64_t, int, int64_t, double, int*);
+template bool jacobi_cluster<zc>(zc*, int, int, int64_t, int, int64_t, double, int*);
 
 }  // namespace ttn

@@ -114,8 +114,7 @@ __global__ void __launch_bounds__(GT) gram_pairs_kernel(const T* __restrict__ X,
 // round-robin over the 64 panel columns (used for the intra-block step, where B is empty).
 template <class T, int ET>
 __global__ void __launch_bounds__(ET) gram_eig_kernel(const T* __restrict__ Gp, int nsplit, int cross_only, double tol,
-                                                      const double* __restrict__ d_frob2, double floor_k, T* __restrict__ Vg, int* __restrict__ skip,
-                                                      unsigned int* __restrict__ d_rotated) {
+                                                      T* __restrict__ Vg, int* __restrict__ skip, unsigned int* __restrict__ d_rotated) {
   constexpr int P = PW + 1;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   T* G = reinterpret_cast<T*>(smem_raw);      // [PW][P]
@@ -126,7 +125,6 @@ __global__ void __launch_bounds__(ET) gram_eig_kernel(const T* __restrict__ Gp, 
   __shared__ int s_any, s_big, s_step[2];
   const int tid = threadIdx.x;
   const double tol2 = tol * tol;
-  const double floor2 = floor_k * d_frob2[0];   // optional noise floor (jacobi.cu JAC_FLOOR2), 0 = off
   const T* gp = Gp + (size_t)blockIdx.x * nsplit * PW * PW;
   for (int idx = tid; idx < PW * PW; idx += ET) {
     T a = t_zero<T>();
@@ -160,7 +158,7 @@ __global__ void __launch_bounds__(ET) gram_eig_kernel(const T* __restrict__ Gp, 
         const double cc = cr * cr + ci * ci;
         double cs = 1.0;
         T sn = t_zero<T>();
-        if (cc > tol2 * fmax(a, 0.0) * fmax(b, 0.0) && a > floor2 && b > floor2 && cc > 1e-290) {
+        if (cc > tol2 * fmax(a, 0.0) * fmax(b, 0.0) && a > 0.0 && b > 0.0 && cc > 1e-290) {
           const double tau = 0.5 * (b - a);
           const double z = tau * tau + cc;
           const double h = z * rsqrt(z);
@@ -329,7 +327,7 @@ __global__ void __launch_bounds__(GT) update_pairs_kernel(T* __restrict__ X, int
 
 // Orthogonalises the n columns of X (m x n, one matrix); returns the number of sweeps, or -1 if the shape is not served.
 template <class T>
-int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2, double fk, int max_sweeps) {
+int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, int max_sweeps) {
   if (n < 2 * PW || m < PW) return -1;
   const int nblk = (n + GB - 1) / GB;
   const int ne = nblk + (nblk & 1);
@@ -348,28 +346,26 @@ int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2
   const int off_diag = (int)hA.size();
   for (int i = 0; i < nblk; ++i) { hA.push_back(i); hB.push_back(-1); }
   const int maxpairs = std::max(ne / 2, nblk);
-  // Several pair groups per step on separate streams: while the (few, latency-bound) inner eigen-sweep CTAs of one group
-  // run, the DMMA Gram / update tiles of the others fill the remaining SMs.  Each group has its own Gram / V / skip buffers
+  // Two pair groups per step on two streams: while the (few, latency-bound) inner eigen-sweep CTAs of one group run, the
+  // DMMA Gram / update tiles of the other fill the remaining SMs.  Each group has its own Gram / V / skip buffers
   // and its own split of the rows sized for ~2 CTAs per SM.
-  constexpr int NGMAX = 4;
-  static cudaStream_t strm[NGMAX] = {nullptr, nullptr, nullptr, nullptr};   // strm[0] is the library stream
-  static cudaEvent_t ev_grp[NGMAX], ev_join = nullptr;
+  constexpr int NG = 2;
+  static cudaStream_t strm[NG] = {nullptr, nullptr};   // strm[0] is the library stream
+  static cudaEvent_t ev_grp[NG], ev_join = nullptr;
   static int strm_dev = -1;   // streams and events belong to a device: rebuild them when ttn_init re-binds the library
   if (ev_join != nullptr && strm_dev != ctx().device) {
-    for (int g = 1; g < NGMAX; ++g) { cudaStreamDestroy(strm[g]); strm[g] = nullptr; }
-    for (int g = 0; g < NGMAX; ++g) cudaEventDestroy(ev_grp[g]);
+    for (int g = 1; g < NG; ++g) { cudaStreamDestroy(strm[g]); strm[g] = nullptr; }
+    for (int g = 0; g < NG; ++g) cudaEventDestroy(ev_grp[g]);
     cudaEventDestroy(ev_join);
     ev_join = nullptr;
   }
   if (ev_join == nullptr) {
     strm_dev = ctx().device;
-    for (int g = 1; g < NGMAX; ++g) TTN_CUDA(cudaStreamCreateWithFlags(&strm[g], cudaStreamNonBlocking));
-    for (int g = 0; g < NGMAX; ++g) TTN_CUDA(cudaEventCreateWithFlags(&ev_grp[g], cudaEventDisableTiming));
+    for (int g = 1; g < NG; ++g) TTN_CUDA(cudaStreamCreateWithFlags(&strm[g], cudaStreamNonBlocking));
+    for (int g = 0; g < NG; ++g) TTN_CUDA(cudaEventCreateWithFlags(&ev_grp[g], cudaEventDisableTiming));
     TTN_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
   }
   strm[0] = ctx().stream;
-  static const int ng_env = getenv("TTN_GRAM_GROUPS") ? atoi(getenv("TTN_GRAM_GROUPS")) : 0;
-  const int NG = std::max(1, std::min(NGMAX, ng_env > 0 ? ng_env : 2));
   const int grpmax = (maxpairs + NG - 1) / NG;
   auto split_for = [&](int cnt, int& ns, int& mcs) {
     ns = std::max(1, std::min((2 * ctx().sm_count + cnt - 1) / std::max(cnt, 1), m / (2 * GK)));
@@ -380,7 +376,7 @@ int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2
   };
   const size_t gp_elems = (size_t)grpmax * 16 * PW * PW;          // <= 16 row splits
   DevBuf gA(sizeof(int) * hA.size()), gB(sizeof(int) * hB.size());
-  DevBuf Gp[NGMAX], Vg[NGMAX], skip[NGMAX], rot(sizeof(unsigned int));
+  DevBuf Gp[NG], Vg[NG], skip[NG], rot(sizeof(unsigned int));
   for (int g = 0; g < NG; ++g) {
     Gp[g].alloc(sizeof(T) * gp_elems);
     Vg[g].alloc(sizeof(T) * (size_t)grpmax * PW * PW);
@@ -407,8 +403,7 @@ int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2
     split_for(cnt, ns, mcs);
     gram_pairs_kernel<T><<<dim3(cnt, ns), GT, smem_g, st>>>(X, m, n, ldx, pa, pb, mcs, Gp[g].as<T>());
     TTN_CHECK_LAUNCH();
-    gram_eig_kernel<T, GE><<<cnt, GE, smem_e, st>>>(Gp[g].as<T>(), ns, cross, tol, frob2, fk, Vg[g].as<T>(), skip[g].as<int>(),
-                                                   rot.as<unsigned int>());
+    gram_eig_kernel<T, GE><<<cnt, GE, smem_e, st>>>(Gp[g].as<T>(), ns, cross, tol, Vg[g].as<T>(), skip[g].as<int>(), rot.as<unsigned int>());
     TTN_CHECK_LAUNCH();
     update_pairs_kernel<T><<<dim3(cnt, (m + UM - 1) / UM), GT, smem_u, st>>>(X, m, n, ldx, pa, pb, Vg[g].as<T>(), skip[g].as<int>());
     TTN_CHECK_LAUNCH();
@@ -451,7 +446,7 @@ int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2
   return sweeps;
 }
 
-template int jacobi_gram<double>(double*, int, int, int64_t, double, const double*, double, int);
-template int jacobi_gram<zc>(zc*, int, int, int64_t, double, const double*, double, int);
+template int jacobi_gram<double>(double*, int, int, int64_t, double, int);
+template int jacobi_gram<zc>(zc*, int, int, int64_t, double, int);
 
 }  // namespace ttn

@@ -389,12 +389,11 @@ template <class T>
 void qr_factor(T* A, int m, int n, int64_t lda, T* tau, int batch, int64_t bA, int64_t btau) {
   const int k = std::min(m, n);
   if (k <= 0 || batch <= 0) return;
-  static const bool smem_panel_env = !(getenv("TTN_QR_SMEM_PANEL") && atoi(getenv("TTN_QR_SMEM_PANEL")) == 0);
   static int attr_dev = -1;   // function attributes are per device (ttn_init may re-bind)
   for (int j0 = 0; j0 < k; j0 += PANEL_NB) {
     // tall single matrix, whole panel inside min(m, n): shared-memory sub-panel kernel
     int SW = 0;
-    if (smem_panel_env && batch == 1 && m - j0 >= 512 && j0 + PANEL_NB <= k)
+    if (batch == 1 && m - j0 >= 512 && j0 + PANEL_NB <= k)
       for (int c : {8, 4, 2})
         if (sizeof(T) * (size_t)c * (m - j0) <= 200 * 1024) { SW = c; break; }
     if (SW > 0) {

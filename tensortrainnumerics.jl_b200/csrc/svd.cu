@@ -11,11 +11,11 @@
 
 namespace ttn {
 
-// TTN_DEBUG_SVD=1 prints one line per factorisation (read once)
-static inline bool debug_svd() {
+bool debug_svd() {
   static const bool on = getenv("TTN_DEBUG_SVD") != nullptr;
   return on;
 }
+
 namespace {
 
 // squared column norms of W (m x n, ld m): one warp per column
@@ -136,9 +136,8 @@ void svd_left(const T* Theta, int p, int q, int64_t rs, int64_t cs, bool conj, S
     // Poor man's column pivoting: order the columns of W = Theta^H (the rows of Theta) by decreasing norm before the unpivoted
     // QR, so that R^H comes out closer to the graded form on which one-sided Jacobi converges fastest (Drmac-Veselic); the
     // row permutation is undone on U Sigma at the end.  DMRG sweep at chi = 1024: 12-17 sweeps per 2048^2 SVD (mean 14.6)
-    // become 12-16 (mean 13.3), Jacobi time -9 %.  TTN_SVD_SORT=0 switches it off.
-    static const bool sort_env = !(getenv("TTN_SVD_SORT") && atoi(getenv("TTN_SVD_SORT")) == 0);
-    const bool sorted = sort_env && batch == 1 && p >= 256;
+    // become 12-16 (mean 13.3), Jacobi time -9 %.
+    const bool sorted = batch == 1 && p >= 256;
     DevBuf dperm;
     if (sorted) {
       DevBuf n2(sizeof(double) * p);
@@ -162,7 +161,7 @@ void svd_left(const T* Theta, int p, int q, int64_t rs, int64_t cs, bool conj, S
       W = std::move(W2);
     }
     DevBuf Rb(sizeof(T) * (size_t)p * p * batch);
-    bool have_r = ctx().use_cholqr && cholqr2<T>(W.as<T>(), q, p, q, bW, Rb.as<T>(), nullptr, 0, 0, batch);
+    const bool have_r = cholqr2<T>(W.as<T>(), q, p, q, bW, Rb.as<T>(), nullptr, 0, 0, batch);
     if (!have_r) {
       DevBuf tau(sizeof(T) * (size_t)p * batch);
       qr_factor<T>(W.as<T>(), q, p, q, tau.as<T>(), batch, bW, p);
@@ -188,7 +187,7 @@ void svd_left(const T* Theta, int p, int q, int64_t rs, int64_t cs, bool conj, S
     range_normalise<T>(W.as<T>(), bW, bW, batch, amax);
     DevBuf Xr(sizeof(T) * (size_t)q * q * batch), Qe(sizeof(T) * (size_t)p * q * batch);
     const int64_t bR = (int64_t)q * q;
-    const bool have_q = ctx().use_cholqr && cholqr2<T>(W.as<T>(), p, q, p, bW, Xr.as<T>(), Qe.as<T>(), p, bW, batch);
+    const bool have_q = cholqr2<T>(W.as<T>(), p, q, p, bW, Xr.as<T>(), Qe.as<T>(), p, bW, batch);
     if (have_q) {
       out.sweeps = jacobi_orth<T>(Xr.as<T>(), q, q, q, out.norms.as<double>(), batch, bR, k);
       GemmArgs g;   // X = Q (R V) = Q * Xr

@@ -278,7 +278,7 @@ void tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, doubl
     const int64_t bA = (int64_t)p * r;
     DevBuf RA(sizeof(T) * (size_t)r * r * batch);
     QA.alloc(sizeof(T) * (size_t)bA * batch);
-    if (!(ctx().use_cholqr && cholqr2<T>(x.core(k), p, r, p, bA, RA.as<T>(), QA.as<T>(), p, bA, batch))) {
+    if (!cholqr2<T>(x.core(k), p, r, p, bA, RA.as<T>(), QA.as<T>(), p, bA, batch)) {
       DevBuf W(sizeof(T) * (size_t)bA * batch), tau(sizeof(T) * (size_t)r * batch);
       TTN_CUDA(cudaMemcpyAsync(W.p, x.cores[k].p, W.bytes, cudaMemcpyDeviceToDevice, ctx().stream));
       qr_factor<T>(W.as<T>(), p, r, p, tau.as<T>(), batch, bA, r);
@@ -699,7 +699,7 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
   int64_t step = 0;
   int ngram = 0;
   bool threw = false;   // a classic step that is fed the output of a declined Gram step may meet non-finite data
-  static const bool dbg = getenv("TTN_DEBUG_SVD") != nullptr;
+  const bool dbg = debug_svd();
   int dbg_prev = 0;
   auto one = [&](int k1, bool l2r) {
     if (threw) return;
@@ -757,7 +757,7 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
   ctx().gram_last_flags = any;
   if (any) {
     ctx().gram_fallbacks++;
-    if (getenv("TTN_DEBUG_SVD")) fprintf(stderr, "[ttn] tt_compress: Gram path declined (flags 0x%x), redoing with the Jacobi path\n", any);
+    if (debug_svd()) fprintf(stderr, "[ttn] tt_compress: Gram path declined (flags 0x%x), redoing with the Jacobi path\n", any);
     for (int k = 0; k < x.d; ++k)
       if (gs.have_orig[k]) x.cores[k] = std::move(gs.orig[k]);
     x.rks = rks0;
@@ -769,13 +769,9 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
   return true;
 }
 
-// src/tt_tools.jl:772-789
+// the plain sweeps of tt_compress!: one Jacobi-SVD bond truncation per step
 template <class T>
-void tt_compress(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
-  ttn_assert(sweeps >= 1, 2, "sweeps must be >= 1");
-  if (ctx().gram_compress && truncerr == 0.0 && x.d >= 2 && max_bond >= 1) {
-    if (tt_compress_gram<T>(x, max_bond, sweeps, sigma_out, sigma_stride)) return;
-  }
+void tt_compress_classic(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
   int64_t step = 0;
   for (int sw = 0; sw < sweeps; ++sw) {
     for (int k = 1; k <= x.d - 1; ++k, ++step)
@@ -785,9 +781,19 @@ void tt_compress(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double
   }
 }
 
+// src/tt_tools.jl:772-789
+template <class T>
+void tt_compress(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
+  ttn_assert(sweeps >= 1, 2, "sweeps must be >= 1");
+  if (ctx().gram_compress && truncerr == 0.0 && x.d >= 2 && max_bond >= 1) {
+    if (tt_compress_gram<T>(x, max_bond, sweeps, sigma_out, sigma_stride)) return;
+  }
+  tt_compress_classic<T>(x, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
+}
+
 // y = tt_compress!(A * x, max_bond; truncerr, sweeps)  (src/tt_operations.jl:101-111 followed by tt_tools.jl:772-789).
 // With truncerr == 0 the product cores are consumed by the L->R pass of the Gram sweep without ever being written to HBM
-// (cfg5: 40.5 MB per vector); otherwise, or when the fast path declines, it is the plain composition of the two calls.
+// (cfg5: 40.5 MB per vector); otherwise, or when the fast path declines, it is tt_apply followed by the plain sweeps.
 template <class T>
 void tt_apply_compress(const TTO<T>& A, const TT<T>& x, TT<T>& y, int64_t max_bond, double truncerr, int sweeps, double* sigma_out,
                        int64_t sigma_stride) {
@@ -811,10 +817,7 @@ void tt_apply_compress(const TTO<T>& A, const TT<T>& x, TT<T>& y, int64_t max_bo
     }
   }
   tt_apply<T>(A, x, y);
-  const bool save = ctx().gram_compress;
-  ctx().gram_compress = false;          // the fast path has just declined this input (or does not apply)
-  try { tt_compress<T>(y, max_bond, truncerr, sweeps, sigma_out, sigma_stride); } catch (...) { ctx().gram_compress = save; throw; }
-  ctx().gram_compress = save;
+  tt_compress_classic<T>(y, max_bond, truncerr, sweeps, sigma_out, sigma_stride);   // the Gram path has declined or does not apply
 }
 
 #define INST(T)                                                                                   \

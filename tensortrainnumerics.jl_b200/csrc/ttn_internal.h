@@ -56,24 +56,19 @@ struct Context {
   bool prof_on = false;    // per-kernel-family CUDA-event timing (bench.py roofline pass only)
   std::vector<ProfRec> prof;
   int last_jacobi_sweeps = 0;  // diagnostics: sweeps used by the most recent Jacobi SVD (batch element 0)
-  bool use_cholqr = true;           // CholeskyQR2 fast path for tall-skinny QR (TTN_NO_CHOLQR=1 disables)
-  bool jacobi_noise_floor = false;  // see JAC_FLOOR2 in jacobi.cu
-  bool use_cluster_jacobi = true;   // single-matrix SVDs on an 8-SM cluster (TTN_NO_CLUSTER_JACOBI=1 disables; A/B timing)
   double flops_gemm = 0.0, flops_heig = 0.0;   // real FLOPs the DMMA GEMMs / the Gram-path eigensolver were asked to execute (roofline accounting)
   long long gram_calls = 0, gram_fallbacks = 0;   // tt_compress! calls that took the Gram path / were redone by the Jacobi path
   int gram_last_flags = 0;
-  bool gemm_bulk = true;            // TMA-staged (cp.async.bulk + mbarrier) big-tile GEMM when the operands allow it; TTN_GEMM_BULK=0 disables
+  bool gemm_bulk = true;            // TMA-staged (cp.async.bulk + mbarrier) big-tile GEMM when the operands allow it
   bool gemm_thin = true;            // streaming kernel for thin right-multiplications (N, K <= 32, shared B): the middle contraction of the local operators
-  int gemm_real_tile = 5;           // Float64 big GEMMs: 5 = 128x64 tile, two CTAs per SM, TMA-staged when the operands allow it (else 3-stage LDGSTS);
-                                    // 0 = the 128x128 one-CTA-per-SM tile of round 1; 1/2/4 = 128x64 with 3/2/4 LDGSTS stages; 3 = 64x64 (A/B timing)
-  int gemm_compact = 1;        // ComplexF64 GEMMs: 1 = 64x64 tile with 2 stages (68 KB, two CTAs per SM, fits next to an eigensolver CTA of another stream); 2/3 = 3/4 stages; 0 = the 64x128 / 64x64 4-stage tiles of round 1
-  bool gram_compress = true;        // Gram path of tt_compress! for truncerr == 0 (heig.cu); TTN_GRAM_COMPRESS=0 disables
+  bool gram_compress = true;        // Gram path of tt_compress! for truncerr == 0 (heig.cu)
   void* host_stage = nullptr;       // pinned staging area of the small device -> host reads (flags, singular values): a pageable
   size_t host_stage_bytes = 0;      // destination would make the read a staged, driver-serialised copy that stalls other host threads
-  int gram_jacobi_min = 640;        // Gram-block Jacobi (DMMA, two streams) for matrices with min(m, n) >= this (measured crossover);
-                                    // TTN_GRAM_JACOBI=1: from 128 columns up, TTN_GRAM_JACOBI=0: never
+  int gram_jacobi_min = 640;        // Gram-block Jacobi (DMMA, two streams) for matrices with min(m, n) >= this (measured crossover)
 };
 Context& ctx();
+/// true when TTN_DEBUG_SVD is set in the environment (read once): the SVD, CholeskyQR2 and Gram-path code then print diagnostics to stderr
+bool debug_svd();
 /// pinned host scratch of at least `bytes` bytes owned by the calling thread's context (valid until the next call)
 void* host_stage(size_t bytes);
 /// blocking device -> host read on the library stream; small reads go through the pinned staging area
@@ -239,10 +234,9 @@ template <class T> void qr_form_q(const T* A, int m, int k, int64_t lda, const T
 template <class T> int jacobi_orth(T* X, int m, int n, int64_t ldx, double* norms, int batch = 1, int64_t bX = 0,
                                    int64_t bnorms = 0);
 // single-matrix path on an 8-CTA cluster (jacobi_cluster.cu); false if the shape is not served
-template <class T> bool jacobi_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, const double* frob2,
-                                       double floor_k, int* d_sweeps);
+template <class T> bool jacobi_cluster(T* X, int m, int n, int64_t ldx, int batch, int64_t bX, double tol, int* d_sweeps);
 // Gram-block Jacobi on the DMMA pipe for one large matrix (jacobi_gram.cu); returns sweeps, or -1 if the shape is not served
-template <class T> int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, const double* frob2, double floor_k, int max_sweeps);
+template <class T> int jacobi_gram(T* X, int m, int n, int64_t ldx, double tol, int max_sweeps);
 // dst (m x r) column j = X[:, perm[j]] * scale[j]   (perm/scale device arrays; per batch strides)
 template <class T> void gather_cols(const T* X, int m, int64_t ldx, const int* perm, const double* scale, int r, T* dst,
                                     int64_t rs, int64_t cs, int batch = 1, int64_t bX = 0, int64_t bperm = 0,

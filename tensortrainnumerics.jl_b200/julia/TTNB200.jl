@@ -161,7 +161,7 @@ function apply_compress(A::TToperator{T}, x::TTvector{T}, max_bond::Int; truncer
     return download(DevTT(out[]))
 end
 
-# run-time switches of the library ("gram_compress", "gemm_bulk", "gram_jacobi_min", "use_cholqr", "use_cluster_jacobi")
+# run-time switches of the library ("gram_compress", "gram_jacobi_min", "gemm_bulk", "gemm_thin", "reset_flops")
 set_option!(key::AbstractString, value::Real) = check(ccall((:ttn_set_option, LIB[]), Cint, (Cstring, Float64), key, value))
 function get_option(key::AbstractString)
     v = Ref{Float64}(0.0)

@@ -201,6 +201,21 @@ def test_sharded_eigsolve_single_rank_matches_dense():
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("bad", [np.nan, np.inf])
+@pytest.mark.parametrize("shape", [(20, 30), (100, 100), (400, 500), (700, 660)])
+def test_svdtrunc_non_finite_input_raises(shape, bad):
+    """One NaN or inf entry is reported as a non-finite singular value, not returned as a result.  The shapes reach each Jacobi
+    engine: one SM (n < 32), the 8-CTA cluster, the cross-CTA block path and the Gram-block path, whose rotation guards skip
+    a pair unless both squared column norms are positive (false for NaN)."""
+    import ttn_b200 as t
+    rng = np.random.default_rng(shape[0] + shape[1])
+    A = rnd(rng, shape, False)
+    A[shape[0] // 3, shape[1] // 2] = bad
+    with pytest.raises(RuntimeError, match="non-finite singular value"):
+        t.svdtrunc(A)
+
+
+@pytest.mark.gpu
 @pytest.mark.parametrize("cond", [1e2, 1e6, 1e12])
 @pytest.mark.parametrize("shape", [(1024, 128), (128, 1024), (300, 64), (96, 96)])
 def test_svdtrunc_across_condition_numbers(shape, cond):
