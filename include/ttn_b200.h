@@ -197,7 +197,8 @@ int ttn_tdvp_params_default(ttn_tdvp_params* p);
 int ttn_tdvp(ttn_tto H, ttn_ttv u0, const ttn_tdvp_params* p, ttn_ttv* u);
 
 /* ---- kernel-level entry points (parity tests, benchmarks) -------------------------------------------- */
-/* strided-batched GEMM on device pointers: C = alpha*op(A)*op(B) + beta*C  (element strides) */
+/* strided-batched GEMM on device pointers: C = alpha*op(A)*op(B) + beta*C  (element strides; batch strides bA/bB/bC, 0 for an
+   operand shared by the whole batch).  Any batch >= 1 is accepted: beyond 65535 products it runs as several launches. */
 int ttn_gemm(int dtype, int M, int N, int K, const void* A, int64_t sAm, int64_t sAk, int conjA, const void* B, int64_t sBk,
              int64_t sBn, int conjB, void* C, int64_t sCm, int64_t sCn, double alpha, double beta, int batch, int64_t bA,
              int64_t bB, int64_t bC);

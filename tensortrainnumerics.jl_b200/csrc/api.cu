@@ -820,7 +820,8 @@ int ttn_gemm(int dtype, int M, int N, int K, const void* A, int64_t sAm, int64_t
   g.B = B; g.sBk = sBk; g.sBn = sBn; g.conjB = conjB != 0;
   g.C = C; g.sCm = sCm; g.sCn = sCn;
   g.alpha = alpha; g.beta = beta;
-  g.batch1 = batch; g.batch2 = 1; g.bA1 = bA; g.bB1 = bB; g.bC1 = bC;
+  // the batch is the outer dimension, which gemm() splits into launches of at most 65535 CTAs along grid.z
+  g.batch1 = 1; g.batch2 = batch; g.bA2 = bA; g.bB2 = bB; g.bC2 = bC;
   if (dtype == TTN_F64) gemm<double>(g); else gemm<zc>(g);
   API_END
 }
