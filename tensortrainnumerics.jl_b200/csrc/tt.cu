@@ -1,6 +1,7 @@
 // TT-level operations on device-resident trains: apply, dot, +, scalar *, orthogonalize, tt_compress!.
 // Each function cites the reference lines it reproduces; the arithmetic is carried by the kernels in
 // gemm.cu / apply.cu / qr.cu / jacobi.cu / elementwise.cu, the host code here only sequences launches.
+#include <functional>
 #include "tt.h"
 
 namespace ttn {
@@ -16,21 +17,31 @@ void tt_copy(const TT<T>& x, TT<T>& y) {
   }
 }
 
-// src/tt_operations.jl:101-111
+// shape of y = A * x (ranks A.rks * x.rks), no core allocated yet
 template <class T>
-void tt_apply(const TTO<T>& A, const TT<T>& x, TT<T>& y) {
-  ttn_assert(A.d == x.d && A.dims == x.dims, 1, "Incompatible dimensions");
+static void product_shape(const TTO<T>& A, const TT<T>& x, TT<T>& y) {
   y.d = x.d; y.batch = x.batch; y.dims = x.dims;
   y.rks.resize(x.d + 1);
   for (int k = 0; k <= x.d; ++k) y.rks[k] = A.rks[k] * x.rks[k];
   y.ot.assign(x.d, 0);
   y.cores.clear();
   y.cores.resize(x.d);
-  for (int k = 0; k < x.d; ++k) {
-    y.alloc_core(k);
-    apply_core<T>(A.core(k), x.core(k), y.core(k), (int)A.dims[k], (int)A.dims[k], (int)A.rks[k], (int)A.rks[k + 1],
-                  (int)x.rks[k], (int)x.rks[k + 1], x.batch, x.core_elems(k), y.core_elems(k));
-  }
+}
+
+// core k of y = A * x   (src/tt_operations.jl:105-108)
+template <class T>
+static void apply_site(const TTO<T>& A, const TT<T>& x, TT<T>& y, int k) {
+  y.alloc_core(k);
+  apply_core<T>(A.core(k), x.core(k), y.core(k), (int)A.dims[k], (int)A.dims[k], (int)A.rks[k], (int)A.rks[k + 1], (int)x.rks[k],
+                (int)x.rks[k + 1], x.batch, x.core_elems(k), y.core_elems(k));
+}
+
+// src/tt_operations.jl:101-111
+template <class T>
+void tt_apply(const TTO<T>& A, const TT<T>& x, TT<T>& y) {
+  ttn_assert(A.d == x.d && A.dims == x.dims, 1, "Incompatible dimensions");
+  product_shape(A, x, y);
+  for (int k = 0; k < x.d; ++k) apply_site(A, x, y, k);
 }
 
 // src/tt_operations.jl:239-250:  M <- A_k^H (B_k M), conj on the first argument
@@ -247,10 +258,53 @@ int rank_tailnorm(const double* s, int len, int64_t max_bond, double truncerr) {
   return r;
 }
 
+// Theta[(s1,alpha),(s2,beta)] = sum_gamma A[s1,alpha,gamma] B[s2,gamma,beta] of bond (k, k+1)     (tt_tools.jl:749)
+template <class T>
+static void two_site_merge(const TT<T>& x, int k, DevBuf& Th) {
+  const int n2 = (int)x.dims[k + 1], p = (int)x.dims[k] * (int)x.rks[k], r = (int)x.rks[k + 1], rr = (int)x.rks[k + 2];
+  GemmArgs g;
+  g.M = p; g.N = rr; g.K = r;
+  g.A = x.cores[k].p; g.sAm = 1; g.sAk = p; g.bA1 = 0; g.bA2 = x.core_elems(k);
+  g.B = x.cores[k + 1].p; g.sBk = n2; g.sBn = (int64_t)n2 * r; g.bB1 = 1; g.bB2 = x.core_elems(k + 1);
+  g.C = Th.p; g.sCm = 1; g.sCn = (int64_t)p * n2; g.bC1 = p; g.bC2 = (int64_t)p * n2 * rr;
+  g.batch1 = n2; g.batch2 = x.batch;
+  gemm<T>(g);
+}
+
+// newB[s2,kappa,beta] = sum_row conj(G2[row,kappa]) Th[row,(s2,beta)] for the rc computed of rn rows: core k+1 of a split bond
+template <class T>
+static void project(const DevBuf& G2, const DevBuf& Th, int pe, int rc, int rn, int n2, int rr, int batch, DevBuf& newB) {
+  GemmArgs g;
+  g.M = rc; g.N = rr; g.K = pe;
+  g.A = G2.p; g.sAm = pe; g.sAk = 1; g.conjA = true; g.bA1 = 0; g.bA2 = (int64_t)pe * rc;
+  g.B = Th.p; g.sBk = 1; g.sBn = (int64_t)pe * n2; g.bB1 = pe; g.bB2 = (int64_t)pe * n2 * rr;
+  g.C = newB.p; g.sCm = n2; g.sCn = (int64_t)n2 * rn; g.bC1 = 1; g.bC2 = (int64_t)n2 * rn * rr;
+  g.batch1 = n2; g.batch2 = batch;
+  gemm<T>(g);
+}
+
+// the cores that replace k and k+1 of a truncated bond, A (p x rn) and B (n2 x rn x rr) per train, and the squared column norms w
+// (rn per train) of a core k = U sqrt(S)
+struct NewBond { DevBuf A, B, w; };
+
+// allocates a NewBond (w only when asked) and zero-fills it when only `computed` < rn columns will be written
+template <class T>
+static NewBond new_bond(int p, int n2, int rn, int rr, int batch, int computed, bool with_w) {
+  NewBond nb;
+  nb.A.alloc(sizeof(T) * (size_t)p * rn * batch);
+  nb.B.alloc(sizeof(T) * (size_t)n2 * rn * rr * batch);
+  if (with_w) nb.w.alloc(sizeof(double) * (size_t)rn * batch);
+  if (computed < rn) {
+    fill<T>(nb.A.as<T>(), (int64_t)p * rn * batch, t_zero<T>());
+    fill<T>(nb.B.as<T>(), (int64_t)n2 * rn * rr * batch, t_zero<T>());
+    if (with_w) TTN_CUDA(cudaMemsetAsync(nb.w.p, 0, nb.w.bytes, ctx().stream));
+  }
+  return nb;
+}
+
 // src/tt_tools.jl:743-768 (without the discarded orthogonalize of :769)
 template <class T>
-void tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, double* sigma_out, int64_t sigma_cap,
-                      std::vector<RetiredCore>* retired) {
+std::pair<DevBuf, DevBuf> tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, double* sigma_out, int64_t sigma_cap) {
   ttn_assert(1 <= k1 && k1 < x.d, 2, "k must be in 1:(N-1)");
   ttn_assert(max_bond >= 1, 2, "max_bond must be >= 1");
   const int k = k1 - 1, batch = x.batch;
@@ -267,13 +321,7 @@ void tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, doubl
   const int pe = factored ? r : p;                   // rows of the matrix that is actually decomposed
   DevBuf Theta(sizeof(T) * (size_t)pe * q * batch), QA;
   if (!factored) {
-    GemmArgs g;  // Theta[(s1,alpha),(s2,beta)] = sum_gamma A[s1,alpha,gamma] B[s2,gamma,beta]     (tt_tools.jl:749)
-    g.M = p; g.N = rr; g.K = r;
-    g.A = x.cores[k].p; g.sAm = 1; g.sAk = p; g.bA1 = 0; g.bA2 = x.core_elems(k);
-    g.B = x.cores[k + 1].p; g.sBk = n2; g.sBn = (int64_t)n2 * r; g.bB1 = 1; g.bB2 = x.core_elems(k + 1);
-    g.C = Theta.p; g.sCm = 1; g.sCn = (int64_t)p * n2; g.bC1 = p; g.bC2 = (int64_t)p * q;
-    g.batch1 = n2; g.batch2 = batch;
-    gemm<T>(g);
+    two_site_merge(x, k, Theta);
   } else {
     const int64_t bA = (int64_t)p * r;
     DevBuf RA(sizeof(T) * (size_t)r * r * batch);
@@ -333,14 +381,10 @@ void tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, doubl
   TTN_CUDA(cudaMemcpyAsync(ds1.p, s1.data(), ds1.bytes, cudaMemcpyHostToDevice, ctx().stream));
   TTN_CUDA(cudaMemcpyAsync(ds2.p, s2.data(), ds2.bytes, cudaMemcpyHostToDevice, ctx().stream));
 
-  DevBuf newA(sizeof(T) * (size_t)p * rn * batch), G2(sizeof(T) * (size_t)pe * rc * batch);
-  DevBuf newB(sizeof(T) * (size_t)n2 * rn * rr * batch);
-  if (rc < rn) {
-    fill<T>(newA.as<T>(), (int64_t)p * rn * batch, t_zero<T>());
-    fill<T>(newB.as<T>(), (int64_t)n2 * rn * rr * batch, t_zero<T>());
-  }
+  NewBond nb = new_bond<T>(p, n2, rn, rr, batch, rc, false);
+  DevBuf G2(sizeof(T) * (size_t)pe * rc * batch);
   if (!factored) {
-    gather_cols<T>(sv.X.as<T>(), p, p, dperm.as<int>(), ds1.as<double>(), rc, newA.as<T>(), 1, p, batch, (int64_t)p * kk, rc,
+    gather_cols<T>(sv.X.as<T>(), p, p, dperm.as<int>(), ds1.as<double>(), rc, nb.A.as<T>(), 1, p, batch, (int64_t)p * kk, rc,
                    (int64_t)p * rn);
   } else {
     DevBuf Us(sizeof(T) * (size_t)pe * rc * batch);   // U' sqrt(S)^{-1}-scaled columns of the small problem
@@ -350,29 +394,18 @@ void tt_bond_truncate(TT<T>& x, int k1, int64_t max_bond, double truncerr, doubl
     g.M = p; g.N = rc; g.K = pe;
     g.A = QA.p; g.sAm = 1; g.sAk = p; g.bA1 = (int64_t)p * r;
     g.B = Us.p; g.sBk = 1; g.sBn = pe; g.bB1 = (int64_t)pe * rc;
-    g.C = newA.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
+    g.C = nb.A.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
     g.batch1 = batch;
     gemm<T>(g);
   }
   gather_cols<T>(sv.X.as<T>(), pe, pe, dperm.as<int>(), ds2.as<double>(), rc, G2.as<T>(), 1, pe, batch, (int64_t)pe * kk, rc,
                  (int64_t)pe * rc);
-  {
-    GemmArgs g;  // newB[s2,kappa,beta] = sum_row conj(G2[row,kappa]) Theta[row,(s2,beta)]
-    g.M = rc; g.N = rr; g.K = pe;
-    g.A = G2.p; g.sAm = pe; g.sAk = 1; g.conjA = true; g.bA1 = 0; g.bA2 = (int64_t)pe * rc;
-    g.B = Theta.p; g.sBk = 1; g.sBn = (int64_t)pe * n2; g.bB1 = pe; g.bB2 = (int64_t)pe * q;
-    g.C = newB.p; g.sCm = n2; g.sCn = (int64_t)n2 * rn; g.bC1 = 1; g.bC2 = (int64_t)n2 * rn * rr;
-    g.batch1 = n2; g.batch2 = batch;
-    gemm<T>(g);
-  }
+  project<T>(G2, Theta, pe, rc, rn, n2, rr, batch, nb.B);
   TTN_CUDA(cudaStreamSynchronize(ctx().stream));
-  if (retired) {
-    retired->push_back(RetiredCore{k, std::move(x.cores[k])});
-    retired->push_back(RetiredCore{k + 1, std::move(x.cores[k + 1])});
-  }
-  x.cores[k] = std::move(newA);
-  x.cores[k + 1] = std::move(newB);
+  std::swap(x.cores[k], nb.A);
+  std::swap(x.cores[k + 1], nb.B);
   x.rks[k + 1] = rn;
+  return {std::move(nb.A), std::move(nb.B)};
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -434,7 +467,6 @@ struct GramSweep {
   std::vector<DevBuf> colw;           // colw[k]: squared column norms of core k (batch x r) while it is U sqrt(S) of bond k
   std::vector<DevBuf> orig;           // input cores (the first buffer replaced per site), alive until the flags are read
   std::vector<char> have_orig;
-  std::vector<RetiredCore> retired;   // cores replaced by classic steps (absorbed into `orig` right after the step)
   DevBuf sigdev;                      // steps x stride singular values of train 0
   std::vector<int> gram_steps;
   int64_t sigma_stride = 0;
@@ -443,14 +475,19 @@ struct GramSweep {
     flags.alloc(sizeof(int) * (size_t)x.batch);
     TTN_CUDA(cudaMemsetAsync(flags.p, 0, flags.bytes, ctx().stream));
   }
-  void replace(int k, DevBuf&& nb) {
-    if (!have_orig[k]) { orig[k] = std::move(x.cores[k]); have_orig[k] = 1; }
-    x.cores[k] = std::move(nb);
+  // a buffer that has left site k: the first one is the input core and is kept for the rollback, later ones are released
+  void retire(int k, DevBuf old) {
+    if (!have_orig[k]) { orig[k] = std::move(old); have_orig[k] = 1; }
   }
-  void absorb_retired() {
-    for (auto& rc : retired)
-      if (!have_orig[rc.k]) { orig[rc.k] = std::move(rc.buf); have_orig[rc.k] = 1; }
-    retired.clear();
+  // the truncated bond replaces cores k and k+1 (no longer a pending product); nb.w, possibly empty, becomes colw[k]
+  void install(int k, NewBond&& nb, int rn) {
+    colw[k] = std::move(nb.w);
+    std::swap(x.cores[k], nb.A);
+    std::swap(x.cores[k + 1], nb.B);
+    retire(k, std::move(nb.A));
+    retire(k + 1, std::move(nb.B));
+    if (lazy) lazy->virt[k + 1] = 0;
+    x.rks[k + 1] = rn;
   }
   // split-K Gram matrix of Th (pe x q, ld pe, batch stride pe*q): partials [nsplit][batch][pe x pe]
   int gram(const T* Th, int pe, int q, DevBuf& Gp) {
@@ -469,25 +506,20 @@ struct GramSweep {
     gemm<T>(g);
     return nsplit;
   }
-  // newB[s2,kappa,beta] = sum_row conj(G2[row,kappa]) Th[row,(s2,beta)]
-  void project(const DevBuf& G2, const DevBuf& Th, int pe, int rc, int rn, int n2, int rr, DevBuf& newB) {
+  // G = V diag(lam) V^H of order n (the sum of nsplit partials sG apart): its top nev eigenpairs, then heig_finalize into out1 /
+  // out2 (and the kept weights into w) with the sweep's flags and this step's sig0.  False when the shape is not served.
+  bool eig_split(const DevBuf& G, int n, int nsplit, int64_t sG, int nev, const double* w_in, T* out1, int64_t ld1, int64_t b1,
+                 T* out2, int64_t ld2, int64_t b2, double* w, int64_t bw, double* sig0) {
     const int batch = x.batch;
-    const int64_t q = (int64_t)n2 * rr;
-    GemmArgs g;
-    g.M = rc; g.N = rr; g.K = pe;
-    g.A = G2.p; g.sAm = pe; g.sAk = 1; g.conjA = true; g.bA1 = 0; g.bA2 = (int64_t)pe * rc;
-    g.B = Th.p; g.sBk = 1; g.sBn = (int64_t)pe * n2; g.bB1 = pe; g.bB2 = (int64_t)pe * q;
-    g.C = newB.p; g.sCm = n2; g.sCn = (int64_t)n2 * rn; g.bC1 = 1; g.bC2 = (int64_t)n2 * rn * rr;
-    g.batch1 = n2; g.batch2 = batch;
-    gemm<T>(g);
+    DevBuf lam(sizeof(double) * (size_t)nev * batch), V(sizeof(T) * (size_t)n * nev * batch);
+    if (!heig_top<T>(G.as<T>(), n, n, (int64_t)n * n, nsplit, sG, nev, batch, lam.as<double>(), V.as<T>(), flags.as<int>()))
+      return false;
+    heig_finalize<T>(V.as<T>(), n, nev, batch, lam.as<double>(), w_in, out1, ld1, b1, out2, ld2, b2, w, bw, sig0, flags.as<int>());
+    return true;
   }
   void materialize(int k) {
     if (!lazy || !lazy->virt[k]) return;
-    const TTO<T>& A = *lazy->A;
-    const TT<T>& v = *lazy->x;
-    x.alloc_core(k);
-    apply_core<T>(A.core(k), v.core(k), x.core(k), (int)A.dims[k], (int)A.dims[k], (int)A.rks[k], (int)A.rks[k + 1], (int)v.rks[k],
-                  (int)v.rks[k + 1], v.batch, v.core_elems(k), x.core_elems(k));
+    apply_site(*lazy->A, *lazy->x, x, k);
     lazy->virt[k] = 0;
   }
   // Theta (p x q) of bond (k, k+1) when core k+1 is still A_{k+1} (x) x_{k+1}:  Z = P x_{k+1} (GEMMs), then the MPO mix
@@ -523,81 +555,14 @@ struct GramSweep {
     }
   }
   // Theta (p x q) of bond (k, k+1), materialised or folded product
-  void theta(int k, bool virt, DevBuf& Th) {
-    const int batch = x.batch;
-    const int n1 = (int)x.dims[k], n2 = (int)x.dims[k + 1];
-    const int rl = (int)x.rks[k], r = (int)x.rks[k + 1], rr = (int)x.rks[k + 2];
-    const int p = n1 * rl, q = n2 * rr;
-    if (virt && (size_t)lazy->A->rks[k + 1] * n2 * n2 * lazy->A->rks[k + 2] * sizeof(T) <= 40 * 1024) {
+  void theta(int k, DevBuf& Th) {
+    const int n2 = (int)x.dims[k + 1];
+    if (lazy && lazy->virt[k + 1] && (size_t)lazy->A->rks[k + 1] * n2 * n2 * lazy->A->rks[k + 2] * sizeof(T) <= 40 * 1024) {
       theta_lazy(k, Th);           // core k+1 stays virtual until the truncated core replaces it
     } else {
       materialize(k + 1);
-      GemmArgs g;  // Theta[(s1,alpha),(s2,beta)] = sum_gamma A[s1,alpha,gamma] B[s2,gamma,beta]     (tt_tools.jl:749)
-      g.M = p; g.N = rr; g.K = r;
-      g.A = x.cores[k].p; g.sAm = 1; g.sAk = p; g.bA1 = 0; g.bA2 = x.core_elems(k);
-      g.B = x.cores[k + 1].p; g.sBk = n2; g.sBn = (int64_t)n2 * r; g.bB1 = 1; g.bB2 = x.core_elems(k + 1);
-      g.C = Th.p; g.sCm = 1; g.sCn = (int64_t)p * n2; g.bC1 = p; g.bC2 = (int64_t)p * q;
-      g.batch1 = n2; g.batch2 = batch;
-      gemm<T>(g);
+      two_site_merge(x, k, Th);
     }
-  }
-  // L->R step of a TALL bond (p > q: the last sites of a train): G = Theta^H Theta = V S^2 V^H (q x q),
-  // core k+1 <- sqrt(S) V^H, core k <- Theta V S^{-1/2} = U sqrt(S)
-  bool step_tall(int k, bool virt, int nev, int rn, double* sig0) {
-    const int batch = x.batch;
-    const int n1 = (int)x.dims[k], n2 = (int)x.dims[k + 1];
-    const int rl = (int)x.rks[k], rr = (int)x.rks[k + 2];
-    const int p = n1 * rl, q = n2 * rr;
-    DevBuf Th(sizeof(T) * (size_t)p * q * batch);
-    theta(k, virt, Th);
-    DevBuf Gp(sizeof(T) * (size_t)q * q * batch);
-    {
-      GemmArgs g;   // G[c, c'] = sum_row conj(Theta[row, c]) Theta[row, c']
-      g.M = q; g.N = q; g.K = p;
-      g.A = Th.p; g.sAm = p; g.sAk = 1; g.conjA = true; g.bA1 = (int64_t)p * q;
-      g.B = Th.p; g.sBk = 1; g.sBn = p; g.bB1 = (int64_t)p * q;
-      g.C = Gp.p; g.sCm = 1; g.sCn = q; g.bC1 = (int64_t)q * q;
-      g.batch1 = batch;
-      gemm<T>(g);
-    }
-    DevBuf lam(sizeof(double) * (size_t)nev * batch), V(sizeof(T) * (size_t)q * nev * batch);
-    if (!heig_top<T>(Gp.as<T>(), q, q, (int64_t)q * q, 1, 0, nev, batch, lam.as<double>(), V.as<T>(), flags.as<int>())) {
-      materialize(k + 1);
-      return false;
-    }
-    DevBuf Vs(sizeof(T) * (size_t)q * nev * batch), Vi(sizeof(T) * (size_t)q * nev * batch), w(sizeof(double) * (size_t)rn * batch);
-    DevBuf newA(sizeof(T) * (size_t)p * rn * batch), newB(sizeof(T) * (size_t)n2 * rn * rr * batch);
-    if (nev < rn) {
-      fill<T>(newA.as<T>(), (int64_t)p * rn * batch, t_zero<T>());
-      fill<T>(newB.as<T>(), (int64_t)n2 * rn * rr * batch, t_zero<T>());
-      TTN_CUDA(cudaMemsetAsync(w.p, 0, w.bytes, ctx().stream));
-    }
-    heig_finalize<T>(V.as<T>(), q, nev, batch, lam.as<double>(), nullptr, Vs.as<T>(), q, (int64_t)q * nev, Vi.as<T>(), q,
-                     (int64_t)q * nev, w.as<double>(), rn, sig0, flags.as<int>());
-    {
-      Copy4 c;   // newB[s2, kappa, beta] = conj(Vs[(s2, beta), kappa])
-      c.n0 = n2; c.s0 = 1; c.d0 = 1;
-      c.n1 = nev; c.s1 = q; c.d1 = n2;
-      c.n2 = rr; c.s2 = n2; c.d2 = (int64_t)n2 * rn;
-      c.n3 = batch; c.s3 = (int64_t)q * nev; c.d3 = (int64_t)n2 * rn * rr;
-      c.conj = true;
-      copy4<T>(Vs.as<T>(), newB.as<T>(), c);
-    }
-    {
-      GemmArgs g;   // core k <- Theta (V S^{-1/2})
-      g.M = p; g.N = nev; g.K = q;
-      g.A = Th.p; g.sAm = 1; g.sAk = p; g.bA1 = (int64_t)p * q;
-      g.B = Vi.p; g.sBk = 1; g.sBn = q; g.bB1 = (int64_t)q * nev;
-      g.C = newA.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
-      g.batch1 = batch;
-      gemm<T>(g);
-    }
-    colw[k] = std::move(w);
-    replace(k, std::move(newA));
-    replace(k + 1, std::move(newB));
-    if (lazy) lazy->virt[k + 1] = 0;
-    x.rks[k + 1] = rn;
-    return true;
   }
   // one bond step; returns false when the shape is not served (caller takes the classic step)
   bool step(int k, bool left_to_right, int64_t step_idx) {
@@ -605,16 +570,14 @@ struct GramSweep {
     materialize(k);
     const int n1 = (int)x.dims[k], n2 = (int)x.dims[k + 1];
     const int rl = (int)x.rks[k], r = (int)x.rks[k + 1], rr = (int)x.rks[k + 2];
-    const int p = n1 * rl, q = n2 * rr, kmin = std::min(p, q);
-    const int rn = (int)std::min<int64_t>(kmin, max_bond);
-    if (rn < 1) return false;
-    const bool have_w = !left_to_right && colw[k].p != nullptr && colw[k].bytes == sizeof(double) * (size_t)r * batch;
+    const int p = n1 * rl, q = n2 * rr;
+    const int rn = (int)std::min<int64_t>(std::min(p, q), max_bond), nev = std::min(rn, r);
     double* sig0 = sigdev.p ? sigdev.as<double>() + step_idx * sigma_stride : nullptr;
-    if (have_w) {
-      materialize(k + 1);
+    if (rn < 1 || ((int64_t)nev > sigma_stride && sig0)) return false;
+    if (!left_to_right && colw[k].p != nullptr && colw[k].bytes == sizeof(double) * (size_t)r * batch) {
+      // R->L: G' = Theta' Theta'^H of Theta' = sqrt(w) B (r x q), the weights w of core k taken from its L->R step
       if (r > heig_max_n<T>() || r > q) return false;
-      const int nev = std::min(rn, r);
-      if ((int64_t)nev > sigma_stride && sig0) return false;
+      materialize(k + 1);
       DevBuf Th(sizeof(T) * (size_t)r * q * batch);
       Copy4 c;   // Th[gamma, s2 + n2*beta] = B[s2, gamma, beta]
       c.n0 = r; c.s0 = n2; c.d0 = 1;
@@ -625,64 +588,88 @@ struct GramSweep {
       diag_scale<T>(Th.as<T>(), r, q, 1, r, colw[k].as<double>(), 1, 0, batch, (int64_t)r * q, r);
       DevBuf Gp;
       const int nsplit = gram(Th.as<T>(), r, q, Gp);
-      DevBuf lam(sizeof(double) * (size_t)nev * batch), W(sizeof(T) * (size_t)r * nev * batch);
-      if (!heig_top<T>(Gp.as<T>(), r, r, (int64_t)r * r, nsplit, (int64_t)batch * r * r, nev, batch, lam.as<double>(), W.as<T>(),
-                       flags.as<int>()))
-        return false;
       DevBuf M1(sizeof(T) * (size_t)r * nev * batch), G2(sizeof(T) * (size_t)r * nev * batch);
-      heig_finalize<T>(W.as<T>(), r, nev, batch, lam.as<double>(), colw[k].as<double>(), M1.as<T>(), r, (int64_t)r * nev, G2.as<T>(),
-                       r, (int64_t)r * nev, nullptr, 0, sig0, flags.as<int>());
-      DevBuf newA(sizeof(T) * (size_t)p * rn * batch), newB(sizeof(T) * (size_t)n2 * rn * rr * batch);
-      if (nev < rn) {
-        fill<T>(newA.as<T>(), (int64_t)p * rn * batch, t_zero<T>());
-        fill<T>(newB.as<T>(), (int64_t)n2 * rn * rr * batch, t_zero<T>());
-      }
+      if (!eig_split(Gp, r, nsplit, (int64_t)batch * r * r, nev, colw[k].as<double>(), M1.as<T>(), r, (int64_t)r * nev, G2.as<T>(), r,
+                     (int64_t)r * nev, nullptr, 0, sig0))
+        return false;
+      NewBond nb = new_bond<T>(p, n2, rn, rr, batch, nev, false);
       GemmArgs g;   // core k <- A M1
       g.M = p; g.N = nev; g.K = r;
       g.A = x.cores[k].p; g.sAm = 1; g.sAk = p; g.bA1 = x.core_elems(k);
       g.B = M1.p; g.sBk = 1; g.sBn = r; g.bB1 = (int64_t)r * nev;
-      g.C = newA.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
+      g.C = nb.A.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
       g.batch1 = batch;
       gemm<T>(g);
-      project(G2, Th, r, nev, rn, n2, rr, newB);
-      colw[k].release();
-      replace(k, std::move(newA));
-      replace(k + 1, std::move(newB));
-      x.rks[k + 1] = rn;
+      project<T>(G2, Th, r, nev, rn, n2, rr, batch, nb.B);
+      install(k, std::move(nb), rn);
       return true;
     }
-    const bool virt = lazy && lazy->virt[k + 1];
-    const int ng = std::min(p, q);                       // order of the Gram matrix: Theta Theta^H (wide) or Theta^H Theta (tall)
-    const bool served = left_to_right && ng <= heig_max_n<T>() && !((int64_t)std::min(rn, r) > sigma_stride && sig0);
-    if (!served) { materialize(k + 1); return false; }
-    const int nev = std::min(rn, r);
-    if (p > q) return step_tall(k, virt, nev, rn, sig0);
+    // L->R: Theta = A B and its Gram matrix of order min(p, q), Theta Theta^H (wide) or Theta^H Theta (tall)
+    if (!left_to_right || std::min(p, q) > heig_max_n<T>()) return false;
     DevBuf Th(sizeof(T) * (size_t)p * q * batch);
-    theta(k, virt, Th);
-    DevBuf Gp;
-    const int nsplit = gram(Th.as<T>(), p, q, Gp);
-    DevBuf lam(sizeof(double) * (size_t)nev * batch), U(sizeof(T) * (size_t)p * nev * batch);
-    if (!heig_top<T>(Gp.as<T>(), p, p, (int64_t)p * p, nsplit, (int64_t)batch * p * p, nev, batch, lam.as<double>(), U.as<T>(),
-                     flags.as<int>()))
-      return false;
-    DevBuf newA(sizeof(T) * (size_t)p * rn * batch), newB(sizeof(T) * (size_t)n2 * rn * rr * batch), G2(sizeof(T) * (size_t)p * nev * batch);
-    DevBuf w(sizeof(double) * (size_t)rn * batch);
-    if (nev < rn) {
-      fill<T>(newA.as<T>(), (int64_t)p * rn * batch, t_zero<T>());
-      fill<T>(newB.as<T>(), (int64_t)n2 * rn * rr * batch, t_zero<T>());
-      TTN_CUDA(cudaMemsetAsync(w.p, 0, w.bytes, ctx().stream));
+    theta(k, Th);
+    NewBond nb;
+    if (p <= q) {
+      DevBuf Gp;
+      const int nsplit = gram(Th.as<T>(), p, q, Gp);
+      nb = new_bond<T>(p, n2, rn, rr, batch, nev, true);
+      DevBuf G2(sizeof(T) * (size_t)p * nev * batch);
+      if (!eig_split(Gp, p, nsplit, (int64_t)batch * p * p, nev, nullptr, nb.A.as<T>(), p, (int64_t)p * rn, G2.as<T>(), p,
+                     (int64_t)p * nev, nb.w.as<double>(), rn, sig0))
+        return false;
+      project<T>(G2, Th, p, nev, rn, n2, rr, batch, nb.B);
+    } else {
+      // a TALL bond (the last sites of a train): G = Theta^H Theta = V S^2 V^H (q x q), core k+1 <- sqrt(S) V^H,
+      // core k <- Theta V S^{-1/2} = U sqrt(S)
+      DevBuf Gp(sizeof(T) * (size_t)q * q * batch);
+      {
+        GemmArgs g;   // G[c, c'] = sum_row conj(Theta[row, c]) Theta[row, c']
+        g.M = q; g.N = q; g.K = p;
+        g.A = Th.p; g.sAm = p; g.sAk = 1; g.conjA = true; g.bA1 = (int64_t)p * q;
+        g.B = Th.p; g.sBk = 1; g.sBn = p; g.bB1 = (int64_t)p * q;
+        g.C = Gp.p; g.sCm = 1; g.sCn = q; g.bC1 = (int64_t)q * q;
+        g.batch1 = batch;
+        gemm<T>(g);
+      }
+      nb = new_bond<T>(p, n2, rn, rr, batch, nev, true);
+      DevBuf Vs(sizeof(T) * (size_t)q * nev * batch), Vi(sizeof(T) * (size_t)q * nev * batch);
+      if (!eig_split(Gp, q, 1, 0, nev, nullptr, Vs.as<T>(), q, (int64_t)q * nev, Vi.as<T>(), q, (int64_t)q * nev, nb.w.as<double>(), rn,
+                     sig0))
+        return false;
+      Copy4 c;   // newB[s2, kappa, beta] = conj(Vs[(s2, beta), kappa])
+      c.n0 = n2; c.s0 = 1; c.d0 = 1;
+      c.n1 = nev; c.s1 = q; c.d1 = n2;
+      c.n2 = rr; c.s2 = n2; c.d2 = (int64_t)n2 * rn;
+      c.n3 = batch; c.s3 = (int64_t)q * nev; c.d3 = (int64_t)n2 * rn * rr;
+      c.conj = true;
+      copy4<T>(Vs.as<T>(), nb.B.as<T>(), c);
+      GemmArgs g;   // core k <- Theta (V S^{-1/2})
+      g.M = p; g.N = nev; g.K = q;
+      g.A = Th.p; g.sAm = 1; g.sAk = p; g.bA1 = (int64_t)p * q;
+      g.B = Vi.p; g.sBk = 1; g.sBn = q; g.bB1 = (int64_t)q * nev;
+      g.C = nb.A.p; g.sCm = 1; g.sCn = p; g.bC1 = (int64_t)p * rn;
+      g.batch1 = batch;
+      gemm<T>(g);
     }
-    heig_finalize<T>(U.as<T>(), p, nev, batch, lam.as<double>(), nullptr, newA.as<T>(), p, (int64_t)p * rn, G2.as<T>(), p,
-                     (int64_t)p * nev, w.as<double>(), rn, sig0, flags.as<int>());
-    project(G2, Th, p, nev, rn, n2, rr, newB);
-    colw[k] = std::move(w);
-    replace(k, std::move(newA));
-    replace(k + 1, std::move(newB));
-    if (lazy) lazy->virt[k + 1] = 0;
-    x.rks[k + 1] = rn;
+    install(k, std::move(nb), rn);
     return true;
   }
 };
+
+// calls step(k, left_to_right, i) for every bond step of `sweeps` sweeps, each bonds k = 1..d-1 (1-based) L->R and then R->L;
+// i numbers the steps from 0 (the row of sigma_out)
+static void for_each_bond_step(int d, int sweeps, const std::function<void(int, bool, int64_t)>& step) {
+  int64_t i = 0;
+  for (int sw = 0; sw < sweeps; ++sw) {
+    for (int k = 1; k <= d - 1; ++k) step(k, true, i++);
+    for (int k = d - 1; k >= 1; --k) step(k, false, i++);
+  }
+}
+
+// the Gram path serves a pure rank cap (truncerr == 0) of a train with at least one bond
+static bool gram_path_applies(int d, int64_t max_bond, double truncerr) {
+  return ctx().gram_compress && truncerr == 0.0 && d >= 2 && max_bond >= 1;
+}
 
 // returns false (x restored to its input) when some eigen-decomposition declined; true when the sweep stands
 template <class T>
@@ -696,12 +683,11 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
     gs.sigdev.alloc(sizeof(double) * (size_t)nsteps * sigma_stride);
     TTN_CUDA(cudaMemsetAsync(gs.sigdev.p, 0, gs.sigdev.bytes, ctx().stream));
   }
-  int64_t step = 0;
   int ngram = 0;
   bool threw = false;   // a classic step that is fed the output of a declined Gram step may meet non-finite data
   const bool dbg = debug_svd();
   int dbg_prev = 0;
-  auto one = [&](int k1, bool l2r) {
+  for_each_bond_step(x.d, sweeps, [&](int k1, bool l2r, int64_t step) {
     if (threw) return;
     if (gs.step(k1 - 1, l2r, step)) {
       gs.gram_steps.push_back((int)step); ++ngram;
@@ -722,19 +708,15 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
       gs.materialize(k1 - 1);
       gs.materialize(k1);
       try {
-        tt_bond_truncate<T>(x, k1, max_bond, 0.0, sigma_out ? sigma_out + step * sigma_stride : nullptr, sigma_stride, &gs.retired);
+        auto old = tt_bond_truncate<T>(x, k1, max_bond, 0.0, sigma_out ? sigma_out + step * sigma_stride : nullptr, sigma_stride);
+        gs.retire(k1 - 1, std::move(old.first));
+        gs.retire(k1, std::move(old.second));
       } catch (const Error&) {
         if (ngram == 0) throw;        // no Gram step before it: the error is the input's
         threw = true;
       }
-      gs.absorb_retired();
     }
-    ++step;
-  };
-  for (int sw = 0; sw < sweeps; ++sw) {
-    for (int k = 1; k <= x.d - 1; ++k) one(k, true);
-    for (int k = x.d - 1; k >= 1; --k) one(k, false);
-  }
+  });
   if (ngram == 0) return true;    // every bond took the classic step: nothing to verify
   ctx().gram_calls++;
   std::vector<int> hf(x.batch);
@@ -772,22 +754,16 @@ bool tt_compress_gram(TT<T>& x, int64_t max_bond, int sweeps, double* sigma_out,
 // the plain sweeps of tt_compress!: one Jacobi-SVD bond truncation per step
 template <class T>
 void tt_compress_classic(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
-  int64_t step = 0;
-  for (int sw = 0; sw < sweeps; ++sw) {
-    for (int k = 1; k <= x.d - 1; ++k, ++step)
-      tt_bond_truncate<T>(x, k, max_bond, truncerr, sigma_out ? sigma_out + step * sigma_stride : nullptr, sigma_stride, nullptr);
-    for (int k = x.d - 1; k >= 1; --k, ++step)
-      tt_bond_truncate<T>(x, k, max_bond, truncerr, sigma_out ? sigma_out + step * sigma_stride : nullptr, sigma_stride, nullptr);
-  }
+  for_each_bond_step(x.d, sweeps, [&](int k, bool, int64_t step) {
+    tt_bond_truncate<T>(x, k, max_bond, truncerr, sigma_out ? sigma_out + step * sigma_stride : nullptr, sigma_stride);
+  });
 }
 
 // src/tt_tools.jl:772-789
 template <class T>
 void tt_compress(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
   ttn_assert(sweeps >= 1, 2, "sweeps must be >= 1");
-  if (ctx().gram_compress && truncerr == 0.0 && x.d >= 2 && max_bond >= 1) {
-    if (tt_compress_gram<T>(x, max_bond, sweeps, sigma_out, sigma_stride)) return;
-  }
+  if (gram_path_applies(x.d, max_bond, truncerr) && tt_compress_gram<T>(x, max_bond, sweeps, sigma_out, sigma_stride)) return;
   tt_compress_classic<T>(x, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
 }
 
@@ -799,13 +775,8 @@ void tt_apply_compress(const TTO<T>& A, const TT<T>& x, TT<T>& y, int64_t max_bo
                        int64_t sigma_stride) {
   ttn_assert(A.d == x.d && A.dims == x.dims, 1, "Incompatible dimensions");
   ttn_assert(sweeps >= 1, 2, "sweeps must be >= 1");
-  if (ctx().gram_compress && truncerr == 0.0 && x.d >= 2 && max_bond >= 1) {
-    y.d = x.d; y.batch = x.batch; y.dims = x.dims;
-    y.rks.resize(x.d + 1);
-    for (int k = 0; k <= x.d; ++k) y.rks[k] = A.rks[k] * x.rks[k];
-    y.ot.assign(x.d, 0);
-    y.cores.clear();
-    y.cores.resize(x.d);
+  if (gram_path_applies(x.d, max_bond, truncerr)) {
+    product_shape(A, x, y);
     LazyProd<T> lazy;
     lazy.A = &A; lazy.x = &x;
     lazy.virt.assign(x.d, 1);
@@ -828,7 +799,7 @@ void tt_apply_compress(const TTO<T>& A, const TT<T>& x, TT<T>& y, int64_t max_bo
   template void tt_add<T>(const TT<T>&, const TT<T>&, TT<T>&);                                    \
   template void tt_scale<T>(const TT<T>&, T, TT<T>&);                                             \
   template void tt_orthogonalize<T>(const TT<T>&, int, TT<T>&);                                   \
-  template void tt_bond_truncate<T>(TT<T>&, int, int64_t, double, double*, int64_t, std::vector<RetiredCore>*); \
+  template std::pair<DevBuf, DevBuf> tt_bond_truncate<T>(TT<T>&, int, int64_t, double, double*, int64_t);   \
   template void tt_compress<T>(TT<T>&, int64_t, double, int, double*, int64_t);
 INST(double)
 INST(zc)

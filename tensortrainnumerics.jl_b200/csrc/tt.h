@@ -35,11 +35,10 @@ template <class T> void tt_scale(const TT<T>& x, T a, TT<T>& y);
 template <class T> void tt_orthogonalize(const TT<T>& x, int center /*1-based*/, TT<T>& y);
 // tail-norm rank rule of src/tt_cross_interpolation.jl:149-166
 int rank_tailnorm(const double* s, int len, int64_t max_bond, double truncerr);
-// a core buffer replaced by a bond step (kept alive by the Gram path of tt_compress! until its verdict is known)
-struct RetiredCore { int k; DevBuf buf; };
+// returns the buffers of the two cores it replaced (k and k+1); dropping them releases them
 template <class T>
-void tt_bond_truncate(TT<T>& x, int k /*1-based*/, int64_t max_bond, double truncerr, double* sigma_out, int64_t sigma_cap,
-                      std::vector<RetiredCore>* retired = nullptr);
+std::pair<DevBuf, DevBuf> tt_bond_truncate(TT<T>& x, int k /*1-based*/, int64_t max_bond, double truncerr, double* sigma_out,
+                                           int64_t sigma_cap);
 template <class T>
 void tt_compress(TT<T>& x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride);
 
