@@ -81,13 +81,12 @@ int ttn_ttv_upload(int dtype, int d, const int64_t* dims, const int64_t* rks, co
                    const void* const* cores, int batch, ttn_ttv* out);
 /* Asynchronous variants for pipelines over batches of trains (cfg5): the copies run on the library's copy stream and overlap
  * the compute stream.  Host buffers must be page-locked and stay valid until the copy has completed.  A handle returned by
- * ttn_ttv_upload_async may be passed to ttn_apply / ttn_apply_compress / ttn_compress / ttn_ttv_download(_async) / ttn_ttv_free
- * right away (they make the compute stream wait for the upload); before any other entry point call ttn_ttv_wait.  After
- * ttn_ttv_download_async the host buffers are valid once ttn_copy_synchronize has returned; ttn_ttv_free may be called at once
- * (the release is ordered after the copy). */
+ * ttn_ttv_upload_async may be passed to any entry point at once: the compute stream waits for the upload, the host does not.
+ * After ttn_ttv_download_async the host buffers are valid once ttn_copy_synchronize has returned.  The in-place entry points
+ * (ttn_compress, ttn_bond_truncate, ttn_swap_sites, ttn_merge_sites_diag, ttn_split_site) and ttn_ttv_free may be called at
+ * once: they replace or release the cores only after the pending download has read them. */
 int ttn_ttv_upload_async(int dtype, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot,
                          const void* const* cores, int batch, ttn_ttv* out);
-int ttn_ttv_wait(ttn_ttv x);
 int ttn_ttv_download_async(ttn_ttv x, void* const* cores);
 int ttn_copy_synchronize(void);
 int ttn_ttv_info(ttn_ttv x, int* dtype, int* d, int* batch);

@@ -69,7 +69,7 @@ def load():
         "ttn_reset_launch_count": [], "ttn_profile": [C.c_int],
         "ttn_profile_read": [C.POINTER(C.c_double), C.POINTER(C.c_longlong)],
         "ttn_ttv_upload": [C.c_int, C.c_int, i64p, i64p, i64p, vpp, C.c_int, vpp],
-        "ttn_ttv_upload_async": [C.c_int, C.c_int, i64p, i64p, i64p, vpp, C.c_int, vpp], "ttn_ttv_wait": [vp],
+        "ttn_ttv_upload_async": [C.c_int, C.c_int, i64p, i64p, i64p, vpp, C.c_int, vpp],
         "ttn_ttv_download_async": [vp, vpp], "ttn_copy_synchronize": [],
         "ttn_ttv_info": [vp, ip, ip, ip], "ttn_ttv_ranks": [vp, i64p], "ttn_ttv_dims": [vp, i64p],
         "ttn_ttv_ot": [vp, i64p], "ttn_ttv_download": [vp, vpp], "ttn_ttv_copy": [vp, vpp],

@@ -1,10 +1,11 @@
 // extern "C" boundary of libttn_b200.so (declared in include/ttn_b200.h).  Converts the library's internal
-// exceptions into status codes; nothing else lives here.
+// exceptions into status codes, and takes the train and operator handles apart and builds new ones.
 #pragma GCC visibility push(default)
 #include "../../include/ttn_b200.h"
 #pragma GCC visibility pop
 #include "tt.h"
 #include "solvers.h"
+#include <memory>
 
 using namespace ttn;
 
@@ -128,6 +129,7 @@ int ttn_profile(int enable) {
 int ttn_profile_read(double* ms, long long* counts) {
   API_BEGIN
   need_init();
+  ttn_assert(ms && counts, TTN_EARG, "null argument");
   Context& c = ctx();
   TTN_CUDA(cudaStreamSynchronize(c.stream));
   for (int i = 0; i < KF_COUNT; ++i) { ms[i] = 0.0; counts[i] = 0; }
@@ -142,49 +144,26 @@ int ttn_profile_read(double* ms, long long* counts) {
 
 // ---------------------------------------------------------------------------------------------------------
 }  // extern "C"
-template <class T>
-static void upload_tt(TT<T>& t, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot, const void* const* cores,
-                      int batch) {
-  t.d = d; t.batch = batch;
-  t.dims.assign(dims, dims + d);
-  t.rks.assign(rks, rks + d + 1);
-  if (ot) t.ot.assign(ot, ot + d); else t.ot.assign(d, 0);
-  t.cores.clear();
-  t.cores.resize(d);
-  for (int k = 0; k < d; ++k) {
-    ttn_assert(dims[k] >= 1 && rks[k] >= 1 && rks[k + 1] >= 1, TTN_EDIM, "upload: dims and ranks must be positive");
-    t.alloc_core(k);
-    TTN_CUDA(cudaMemcpyAsync(t.cores[k].p, cores[k], t.cores[k].bytes, cudaMemcpyHostToDevice, ctx().stream));
-  }
-  TTN_CUDA(cudaStreamSynchronize(ctx().stream));
-}
-extern "C" {
-
-int ttn_ttv_upload(int dtype, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot, const void* const* cores,
-                   int batch, ttn_ttv* out) {
-  API_BEGIN
-  need_init();
-  ttn_assert(d >= 1 && batch >= 1 && out, TTN_EARG, "upload: bad arguments");
-  ttn_assert(dtype == TTN_F64 || dtype == TTN_C128, TTN_EARG, "upload: bad dtype");
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = dtype;
-  try {
-    if (dtype == TTN_F64) upload_tt(h->r, d, dims, rks, ot, cores, batch);
-    else upload_tt(h->c, d, dims, rks, ot, cores, batch);
-  } catch (...) { delete h; throw; }
-  *out = h;
-  API_END
-}
-
-#define TTV_FIELD(x, f) ((x)->dtype == TTN_F64 ? (x)->r.f : (x)->c.f)
-
-}  // extern "C"
 static cudaStream_t copy_stream() {
   Context& c = ctx();
   if (!c.copy_stream) TTN_CUDA(cudaStreamCreateWithFlags(&c.copy_stream, cudaStreamNonBlocking));
   return c.copy_stream;
 }
-// the compute stream waits for a pending asynchronous upload of x (no host synchronisation)
+// the copy stream waits until the compute stream has reached this point (no host synchronisation)
+static void copy_stream_follows_compute() {
+  cudaEvent_t ev;
+  TTN_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  TTN_CUDA(cudaEventRecord(ev, ctx().stream));
+  TTN_CUDA(cudaStreamWaitEvent(copy_stream(), ev, 0));
+  cudaEventDestroy(ev);
+}
+// `ev` (re)recorded at the current end of the copy stream
+static void record_on_copy_stream(cudaEvent_t& ev) {
+  if (ev) cudaEventDestroy(ev);
+  ev = nullptr;
+  TTN_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+  TTN_CUDA(cudaEventRecord(ev, copy_stream()));
+}
 namespace {
 struct DeferredRelease {
   cudaEvent_t ev;
@@ -226,83 +205,111 @@ ttn_ttv_s::~ttn_ttv_s() {
       cudaGetLastError();
       DeferredRelease d;
       d.ev = busy;
-      d.bufs = std::move(dtype == TTN_F64 ? r.cores : c.cores);
+      d.bufs = visit([](auto& t) { return std::move(t.cores); });
       deferred().v.push_back(std::move(d));
     }
   }
   ttn::drain_deferred_releases(false);
 }
 
-static void await_ready(ttn_ttv x) {
-  if (x && x->ready) {
+// The two ways an entry point takes a train whose cores it touches.  Neither makes the host wait.
+//   read_ttv:  the compute stream waits for a pending ttn_ttv_upload_async of x, so such a handle may go anywhere at once.
+//   write_ttv: for the entry points that replace the cores in place; the compute stream also waits for a pending
+//              ttn_ttv_download_async of x, so that the old cores go back to the block cache only after the copy engine
+//              has read them.
+static ttn_ttv_s& read_ttv(ttn_ttv x) {
+  ttn_assert(x != nullptr, TTN_EARG, "null handle");
+  if (x->ready) {
     TTN_CUDA(cudaStreamWaitEvent(ctx().stream, x->ready, 0));
     cudaEventDestroy(x->ready);
     x->ready = nullptr;
   }
+  return *x;
+}
+static ttn_ttv_s& write_ttv(ttn_ttv x) {
+  ttn_ttv_s& h = read_ttv(x);
+  if (h.busy) TTN_CUDA(cudaStreamWaitEvent(ctx().stream, h.busy, 0));
+  return h;
+}
+// an empty result train of element type `dtype`; the entry point hands it out with `*out = h.release()`
+static std::unique_ptr<ttn_ttv_s> new_ttv(int dtype) {
+  with_dtype(dtype, [](auto) {});
+  auto h = std::make_unique<ttn_ttv_s>();
+  h->dtype = dtype;
+  return h;
+}
+// a train shaped from the caller's arrays, its cores allocated but not yet filled
+static std::unique_ptr<ttn_ttv_s> alloc_ttv(int dtype, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot,
+                                            int batch) {
+  ttn_assert(d >= 1 && batch >= 1 && dims && rks, TTN_EARG, "upload: bad arguments");
+  auto h = new_ttv(dtype);
+  h->visit([&](auto& t) {
+    t.d = d; t.batch = batch;
+    t.dims.assign(dims, dims + d);
+    t.rks.assign(rks, rks + d + 1);
+    if (ot) t.ot.assign(ot, ot + d); else t.ot.assign(d, 0);
+    t.cores.resize(d);
+    for (int k = 0; k < d; ++k) {
+      ttn_assert(dims[k] >= 1 && rks[k] >= 1 && rks[k + 1] >= 1, TTN_EDIM, "upload: dims and ranks must be positive");
+      t.alloc_core(k);
+    }
+  });
+  return h;
+}
+// every core of a train or operator between the device and the caller's host arrays, queued on `s`
+template <class H>
+static void copy_cores(H& x, void* const* host, cudaMemcpyKind kind, cudaStream_t s) {
+  ttn_assert(host != nullptr, TTN_EARG, "null argument");
+  x.visit([&](auto& t) {
+    for (int k = 0; k < t.d; ++k) {
+      void* dev = t.cores[k].p;
+      const bool up = kind == cudaMemcpyHostToDevice;
+      TTN_CUDA(cudaMemcpyAsync(up ? dev : host[k], up ? host[k] : dev, t.cores[k].bytes, kind, s));
+    }
+  });
+}
+// rks / dims / ot of a handle into the caller's array
+template <class H, class F>
+static void copy_shape(H* x, int64_t* out, F field) {
+  ttn_assert(x && out, TTN_EARG, "null argument");
+  x->visit([&](auto& t) {
+    const std::vector<int64_t>& v = field(t);
+    std::copy(v.begin(), v.end(), out);
+  });
 }
 extern "C" {
 
+int ttn_ttv_upload(int dtype, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot, const void* const* cores,
+                   int batch, ttn_ttv* out) {
+  API_BEGIN
+  need_init();
+  ttn_assert(out != nullptr, TTN_EARG, "upload: bad arguments");
+  auto h = alloc_ttv(dtype, d, dims, rks, ot, batch);
+  copy_cores(*h, const_cast<void* const*>(cores), cudaMemcpyHostToDevice, ctx().stream);
+  TTN_CUDA(cudaStreamSynchronize(ctx().stream));
+  *out = h.release();
+  API_END
+}
 int ttn_ttv_upload_async(int dtype, int d, const int64_t* dims, const int64_t* rks, const int64_t* ot, const void* const* cores,
                          int batch, ttn_ttv* out) {
   API_BEGIN
   need_init();
-  ttn_assert(d >= 1 && batch >= 1 && out, TTN_EARG, "upload: bad arguments");
-  ttn_assert(dtype == TTN_F64 || dtype == TTN_C128, TTN_EARG, "upload: bad dtype");
+  ttn_assert(out != nullptr, TTN_EARG, "upload: bad arguments");
   drain_deferred_releases(false);
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = dtype;
-  try {
-    auto setup = [&](auto& t) {
-      t.d = d; t.batch = batch;
-      t.dims.assign(dims, dims + d);
-      t.rks.assign(rks, rks + d + 1);
-      if (ot) t.ot.assign(ot, ot + d); else t.ot.assign(d, 0);
-      t.cores.clear();
-      t.cores.resize(d);
-      for (int k = 0; k < d; ++k) {
-        ttn_assert(dims[k] >= 1 && rks[k] >= 1 && rks[k + 1] >= 1, TTN_EDIM, "upload: dims and ranks must be positive");
-        t.alloc_core(k);
-      }
-      // the stream-ordered allocations become usable on the copy stream once the compute stream reaches this point
-      cudaEvent_t ev;
-      TTN_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-      TTN_CUDA(cudaEventRecord(ev, ctx().stream));
-      TTN_CUDA(cudaStreamWaitEvent(copy_stream(), ev, 0));
-      cudaEventDestroy(ev);
-      for (int k = 0; k < d; ++k)
-        TTN_CUDA(cudaMemcpyAsync(t.cores[k].p, cores[k], t.cores[k].bytes, cudaMemcpyHostToDevice, copy_stream()));
-    };
-    if (dtype == TTN_F64) setup(h->r); else setup(h->c);
-    TTN_CUDA(cudaEventCreateWithFlags(&h->ready, cudaEventDisableTiming));
-    TTN_CUDA(cudaEventRecord(h->ready, copy_stream()));
-  } catch (...) { delete h; throw; }
-  *out = h;
-  API_END
-}
-int ttn_ttv_wait(ttn_ttv x) {
-  API_BEGIN
-  need_init();
-  await_ready(x);
+  auto h = alloc_ttv(dtype, d, dims, rks, ot, batch);
+  copy_stream_follows_compute();   // the stream-ordered allocations become usable on the copy stream
+  copy_cores(*h, const_cast<void* const*>(cores), cudaMemcpyHostToDevice, copy_stream());
+  record_on_copy_stream(h->ready);
+  *out = h.release();
   API_END
 }
 int ttn_ttv_download_async(ttn_ttv x, void* const* cores) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  await_ready(x);
-  cudaEvent_t ev;
-  TTN_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-  TTN_CUDA(cudaEventRecord(ev, ctx().stream));            // everything queued on the compute stream so far has produced x
-  TTN_CUDA(cudaStreamWaitEvent(copy_stream(), ev, 0));
-  cudaEventDestroy(ev);
-  const int d = TTV_FIELD(x, d);
-  for (int k = 0; k < d; ++k) {
-    const DevBuf& b = x->dtype == TTN_F64 ? x->r.cores[k] : x->c.cores[k];
-    TTN_CUDA(cudaMemcpyAsync(cores[k], b.p, b.bytes, cudaMemcpyDeviceToHost, copy_stream()));
-  }
-  if (x->busy) cudaEventDestroy(x->busy);
-  TTN_CUDA(cudaEventCreateWithFlags(&x->busy, cudaEventDisableTiming));
-  TTN_CUDA(cudaEventRecord(x->busy, copy_stream()));
+  ttn_ttv_s& h = read_ttv(x);
+  copy_stream_follows_compute();   // everything queued on the compute stream so far has produced x
+  copy_cores(h, cores, cudaMemcpyDeviceToHost, copy_stream());
+  record_on_copy_stream(h.busy);
   API_END
 }
 int ttn_copy_synchronize(void) {
@@ -317,67 +324,53 @@ int ttn_ttv_info(ttn_ttv x, int* dtype, int* d, int* batch) {
   API_BEGIN
   ttn_assert(x != nullptr, TTN_EARG, "null handle");
   if (dtype) *dtype = x->dtype;
-  if (d) *d = TTV_FIELD(x, d);
-  if (batch) *batch = TTV_FIELD(x, batch);
+  x->visit([&](auto& t) {
+    if (d) *d = t.d;
+    if (batch) *batch = t.batch;
+  });
   API_END
 }
 int ttn_ttv_ranks(ttn_ttv x, int64_t* rks) {
   API_BEGIN
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  const auto& v = TTV_FIELD(x, rks);
-  std::copy(v.begin(), v.end(), rks);
+  copy_shape(x, rks, [](auto& t) -> auto& { return t.rks; });
   API_END
 }
 int ttn_ttv_dims(ttn_ttv x, int64_t* dims) {
   API_BEGIN
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  const auto& v = TTV_FIELD(x, dims);
-  std::copy(v.begin(), v.end(), dims);
+  copy_shape(x, dims, [](auto& t) -> auto& { return t.dims; });
   API_END
 }
 int ttn_ttv_ot(ttn_ttv x, int64_t* ot) {
   API_BEGIN
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  const auto& v = TTV_FIELD(x, ot);
-  std::copy(v.begin(), v.end(), ot);
+  copy_shape(x, ot, [](auto& t) -> auto& { return t.ot; });
   API_END
 }
 int ttn_ttv_download(ttn_ttv x, void* const* cores) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  await_ready(x);
-  const int d = TTV_FIELD(x, d);
-  for (int k = 0; k < d; ++k) {
-    const DevBuf& b = x->dtype == TTN_F64 ? x->r.cores[k] : x->c.cores[k];
-    TTN_CUDA(cudaMemcpyAsync(cores[k], b.p, b.bytes, cudaMemcpyDeviceToHost, ctx().stream));
-  }
+  copy_cores(read_ttv(x), cores, cudaMemcpyDeviceToHost, ctx().stream);
   TTN_CUDA(cudaStreamSynchronize(ctx().stream));
   API_END
 }
 int ttn_ttv_copy(ttn_ttv x, ttn_ttv* out) {
   API_BEGIN
   need_init();
-  ttn_assert(x && out, TTN_EARG, "null handle");
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_copy(x->r, h->r); else tt_copy(x->c, h->c);
-  } catch (...) { delete h; throw; }
-  *out = h;
+  ttn_assert(out != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_copy(xs.as<T>(), h->as<T>()); });
+  *out = h.release();
   API_END
 }
 int ttn_ttv_complex(ttn_ttv x, ttn_ttv* out) {
   API_BEGIN
   need_init();
-  ttn_assert(x && out, TTN_EARG, "null handle");
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = TTN_C128;
-  try {
-    if (x->dtype == TTN_C128) tt_copy(x->c, h->c);
-    else tt_to_complex(x->r, h->c);
-  } catch (...) { delete h; throw; }
-  *out = h;
+  ttn_assert(out != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  auto h = new_ttv(TTN_C128);
+  if (xs.dtype == TTN_C128) tt_copy(xs.as<zc>(), h->as<zc>());
+  else tt_to_complex(xs.as<double>(), h->as<zc>());
+  *out = h.release();
   API_END
 }
 int ttn_ttv_free(ttn_ttv x) {
@@ -386,76 +379,61 @@ int ttn_ttv_free(ttn_ttv x) {
   API_END
 }
 
-}  // extern "C"
-template <class T>
-static void upload_tto(TTO<T>& t, int d, const int64_t* dims, const int64_t* rks, const void* const* cores) {
-  t.d = d;
-  t.dims.assign(dims, dims + d);
-  t.rks.assign(rks, rks + d + 1);
-  t.cores.clear();
-  t.cores.resize(d);
-  for (int k = 0; k < d; ++k) {
-    t.cores[k].alloc(sizeof(T) * (size_t)(dims[k] * dims[k] * rks[k] * rks[k + 1]));
-    TTN_CUDA(cudaMemcpyAsync(t.cores[k].p, cores[k], t.cores[k].bytes, cudaMemcpyHostToDevice, ctx().stream));
-  }
-  TTN_CUDA(cudaStreamSynchronize(ctx().stream));
-}
-extern "C" {
 int ttn_tto_upload(int dtype, int d, const int64_t* dims, const int64_t* rks, const void* const* cores, ttn_tto* out) {
   API_BEGIN
   need_init();
-  ttn_assert(d >= 1 && out, TTN_EARG, "upload: bad arguments");
-  ttn_assert(dtype == TTN_F64 || dtype == TTN_C128, TTN_EARG, "upload: bad dtype");
-  ttn_tto h = new ttn_tto_s();
+  ttn_assert(d >= 1 && dims && rks && out, TTN_EARG, "upload: bad arguments");
+  auto h = std::make_unique<ttn_tto_s>();
   h->dtype = dtype;
-  try {
-    if (dtype == TTN_F64) upload_tto(h->r, d, dims, rks, cores); else upload_tto(h->c, d, dims, rks, cores);
-  } catch (...) { delete h; throw; }
-  *out = h;
+  with_dtype(dtype, [&](auto tag) {
+    using T = decltype(tag);
+    TTO<T>& t = h->as<T>();
+    t.d = d;
+    t.dims.assign(dims, dims + d);
+    t.rks.assign(rks, rks + d + 1);
+    t.cores.resize(d);
+    for (int k = 0; k < d; ++k) {
+      ttn_assert(dims[k] >= 1 && rks[k] >= 1 && rks[k + 1] >= 1, TTN_EDIM, "upload: dims and ranks must be positive");
+      t.cores[k].alloc(sizeof(T) * (size_t)(dims[k] * dims[k] * rks[k] * rks[k + 1]));
+    }
+  });
+  copy_cores(*h, const_cast<void* const*>(cores), cudaMemcpyHostToDevice, ctx().stream);
+  TTN_CUDA(cudaStreamSynchronize(ctx().stream));
+  *out = h.release();
   API_END
 }
 int ttn_tto_complex(ttn_tto A, ttn_tto* out) {
   API_BEGIN
   need_init();
   ttn_assert(A && out, TTN_EARG, "null handle");
-  ttn_tto h = new ttn_tto_s();
+  auto h = std::make_unique<ttn_tto_s>();
   h->dtype = TTN_C128;
-  try {
-    if (A->dtype == TTN_C128) tto_copy(A->c, h->c); else tto_to_complex(A->r, h->c);
-  } catch (...) { delete h; throw; }
-  *out = h;
+  if (A->dtype == TTN_C128) tto_copy(A->as<zc>(), h->as<zc>()); else tto_to_complex(A->as<double>(), h->as<zc>());
+  *out = h.release();
   API_END
 }
 int ttn_tto_info(ttn_tto A, int* dtype, int* d) {
   API_BEGIN
   ttn_assert(A != nullptr, TTN_EARG, "null handle");
   if (dtype) *dtype = A->dtype;
-  if (d) *d = A->dtype == TTN_F64 ? A->r.d : A->c.d;
+  if (d) *d = A->visit([](auto& t) { return t.d; });
   API_END
 }
 int ttn_tto_ranks(ttn_tto A, int64_t* rks) {
   API_BEGIN
-  ttn_assert(A && rks, TTN_EARG, "null handle");
-  const auto& v = A->dtype == TTN_F64 ? A->r.rks : A->c.rks;
-  std::copy(v.begin(), v.end(), rks);
+  copy_shape(A, rks, [](auto& t) -> auto& { return t.rks; });
   API_END
 }
 int ttn_tto_dims(ttn_tto A, int64_t* dims) {
   API_BEGIN
-  ttn_assert(A && dims, TTN_EARG, "null handle");
-  const auto& v = A->dtype == TTN_F64 ? A->r.dims : A->c.dims;
-  std::copy(v.begin(), v.end(), dims);
+  copy_shape(A, dims, [](auto& t) -> auto& { return t.dims; });
   API_END
 }
 int ttn_tto_download(ttn_tto A, void* const* cores) {
   API_BEGIN
   need_init();
-  ttn_assert(A && cores, TTN_EARG, "null handle");
-  const int d = A->dtype == TTN_F64 ? A->r.d : A->c.d;
-  for (int k = 0; k < d; ++k) {
-    const DevBuf& b = A->dtype == TTN_F64 ? A->r.cores[k] : A->c.cores[k];
-    TTN_CUDA(cudaMemcpyAsync(cores[k], b.p, b.bytes, cudaMemcpyDeviceToHost, ctx().stream));
-  }
+  ttn_assert(A != nullptr, TTN_EARG, "null handle");
+  copy_cores(*A, cores, cudaMemcpyDeviceToHost, ctx().stream);
   TTN_CUDA(cudaStreamSynchronize(ctx().stream));
   API_END
 }
@@ -471,124 +449,105 @@ static void same_dtype(int a, int b) { ttn_assert(a == b, TTN_EDIM, "element typ
 int ttn_apply(ttn_tto A, ttn_ttv x, ttn_ttv* y) {
   API_BEGIN
   need_init();
-  ttn_assert(A && x && y, TTN_EARG, "null handle");
-  same_dtype(A->dtype, x->dtype);
-  await_ready(x);
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_apply(A->r, x->r, h->r); else tt_apply(A->c, x->c, h->c);
-  } catch (...) { delete h; throw; }
-  *y = h;
+  ttn_assert(A && y, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  same_dtype(A->dtype, xs.dtype);
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_apply(A->as<T>(), xs.as<T>(), h->as<T>()); });
+  *y = h.release();
   API_END
 }
 int ttn_dot(ttn_ttv a, ttn_ttv b, double* out) {
   API_BEGIN
   need_init();
-  ttn_assert(a && b && out, TTN_EARG, "null handle");
-  same_dtype(a->dtype, b->dtype);
-  if (a->dtype == TTN_F64) {
-    std::vector<double> v;
-    tt_dot(a->r, b->r, v);
-    for (size_t i = 0; i < v.size(); ++i) { out[2 * i] = v[i]; out[2 * i + 1] = 0.0; }
-  } else {
-    std::vector<zc> v;
-    tt_dot(a->c, b->c, v);
-    for (size_t i = 0; i < v.size(); ++i) { out[2 * i] = v[i].x; out[2 * i + 1] = v[i].y; }
-  }
+  ttn_assert(out != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& as = read_ttv(a);
+  ttn_ttv_s& bs = read_ttv(b);
+  same_dtype(as.dtype, bs.dtype);
+  with_dtype(as.dtype, [&](auto t) {
+    using T = decltype(t);
+    std::vector<T> v;
+    tt_dot(as.as<T>(), bs.as<T>(), v);
+    for (size_t i = 0; i < v.size(); ++i) { out[2 * i] = t_real(v[i]); out[2 * i + 1] = t_imag(v[i]); }
+  });
   API_END
 }
 int ttn_norm(ttn_ttv a, double* out) {
   API_BEGIN
   need_init();
-  ttn_assert(a && out, TTN_EARG, "null handle");
-  if (a->dtype == TTN_F64) {
-    std::vector<double> v;
-    tt_dot(a->r, a->r, v);
-    for (size_t i = 0; i < v.size(); ++i) out[i] = std::sqrt(v[i] > 0 ? v[i] : 0.0);
-  } else {
-    std::vector<zc> v;
-    tt_dot(a->c, a->c, v);
-    for (size_t i = 0; i < v.size(); ++i) out[i] = std::sqrt(v[i].x > 0 ? v[i].x : 0.0);
-  }
+  ttn_assert(out != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& as = read_ttv(a);
+  with_dtype(as.dtype, [&](auto t) {
+    using T = decltype(t);
+    std::vector<T> v;
+    tt_dot(as.as<T>(), as.as<T>(), v);
+    for (size_t i = 0; i < v.size(); ++i) out[i] = std::sqrt(t_real(v[i]) > 0 ? t_real(v[i]) : 0.0);
+  });
   API_END
 }
 int ttn_add(ttn_ttv x, ttn_ttv y, ttn_ttv* z) {
   API_BEGIN
   need_init();
-  ttn_assert(x && y && z, TTN_EARG, "null handle");
-  same_dtype(x->dtype, y->dtype);
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_add(x->r, y->r, h->r); else tt_add(x->c, y->c, h->c);
-  } catch (...) { delete h; throw; }
-  *z = h;
+  ttn_assert(z != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  ttn_ttv_s& ys = read_ttv(y);
+  same_dtype(xs.dtype, ys.dtype);
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_add(xs.as<T>(), ys.as<T>(), h->as<T>()); });
+  *z = h.release();
   API_END
 }
 int ttn_scale(ttn_ttv x, double re, double im, ttn_ttv* y) {
   API_BEGIN
   need_init();
-  ttn_assert(x && y, TTN_EARG, "null handle");
-  ttn_assert(x->dtype == TTN_C128 || im == 0.0, TTN_EARG, "complex scalar on a real TT (promote first)");
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_scale(x->r, re, h->r); else tt_scale(x->c, make_cuDoubleComplex(re, im), h->c);
-  } catch (...) { delete h; throw; }
-  *y = h;
+  ttn_assert(y != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  ttn_assert(xs.dtype == TTN_C128 || im == 0.0, TTN_EARG, "complex scalar on a real TT (promote first)");
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_scale(xs.as<T>(), t_from<T>(re, im), h->as<T>()); });
+  *y = h.release();
   API_END
 }
 int ttn_orthogonalize(ttn_ttv x, int center, ttn_ttv* y) {
   API_BEGIN
   need_init();
-  ttn_assert(x && y, TTN_EARG, "null handle");
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_orthogonalize(x->r, center, h->r); else tt_orthogonalize(x->c, center, h->c);
-  } catch (...) { delete h; throw; }
-  *y = h;
+  ttn_assert(y != nullptr, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_orthogonalize(xs.as<T>(), center, h->as<T>()); });
+  *y = h.release();
   API_END
 }
 int ttn_compress(ttn_ttv x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  await_ready(x);
-  if (x->dtype == TTN_F64) tt_compress(x->r, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
-  else tt_compress(x->c, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
+  write_ttv(x).visit([&](auto& t) { tt_compress(t, max_bond, truncerr, sweeps, sigma_out, sigma_stride); });
   API_END
 }
 int ttn_apply_compress(ttn_tto A, ttn_ttv x, int64_t max_bond, double truncerr, int sweeps, double* sigma_out, int64_t sigma_stride,
                        ttn_ttv* y) {
   API_BEGIN
   need_init();
-  ttn_assert(A && x && y, TTN_EARG, "null handle");
-  same_dtype(A->dtype, x->dtype);
-  await_ready(x);
-  ttn_ttv h = new ttn_ttv_s();
-  h->dtype = x->dtype;
-  try {
-    if (x->dtype == TTN_F64) tt_apply_compress(A->r, x->r, h->r, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
-    else tt_apply_compress(A->c, x->c, h->c, max_bond, truncerr, sweeps, sigma_out, sigma_stride);
-  } catch (...) { delete h; throw; }
-  *y = h;
+  ttn_assert(A && y, TTN_EARG, "null handle");
+  ttn_ttv_s& xs = read_ttv(x);
+  same_dtype(A->dtype, xs.dtype);
+  auto h = new_ttv(xs.dtype);
+  with_dtype(xs.dtype, [&](auto t) {
+    using T = decltype(t);
+    tt_apply_compress(A->as<T>(), xs.as<T>(), h->as<T>(), max_bond, truncerr, sweeps, sigma_out, sigma_stride);
+  });
+  *y = h.release();
   API_END
 }
 int ttn_bond_truncate(ttn_ttv x, int k, int64_t max_bond, double truncerr, ttn_ttv* y) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  if (x->dtype == TTN_F64) tt_bond_truncate(x->r, k, max_bond, truncerr, nullptr, 0);
-  else tt_bond_truncate(x->c, k, max_bond, truncerr, nullptr, 0);
+  ttn_ttv_s& xs = write_ttv(x);
+  xs.visit([&](auto& t) { tt_bond_truncate(t, k, max_bond, truncerr, nullptr, 0); });
   if (y) {
-    ttn_ttv h = new ttn_ttv_s();
-    h->dtype = x->dtype;
-    try {
-      if (x->dtype == TTN_F64) tt_orthogonalize(x->r, k, h->r); else tt_orthogonalize(x->c, k, h->c);
-    } catch (...) { delete h; throw; }
-    *y = h;
+    auto h = new_ttv(xs.dtype);
+    with_dtype(xs.dtype, [&](auto t) { using T = decltype(t); tt_orthogonalize(xs.as<T>(), k, h->as<T>()); });
+    *y = h.release();
   }
   API_END
 }
@@ -596,26 +555,21 @@ int ttn_bond_truncate(ttn_ttv x, int k, int64_t max_bond, double truncerr, ttn_t
 int ttn_swap_sites(ttn_ttv x, int k, int mode, int64_t max_bond, double tol) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
   ttn_assert(mode == 0 || mode == 1, TTN_EARG, "mode must be 0 (relative threshold) or 1 (tail norm)");
-  if (x->dtype == TTN_F64) tt_swap_sites(x->r, k, mode, max_bond, tol);
-  else tt_swap_sites(x->c, k, mode, max_bond, tol);
+  write_ttv(x).visit([&](auto& t) { tt_swap_sites(t, k, mode, max_bond, tol); });
   API_END
 }
 int ttn_merge_sites_diag(ttn_ttv x, int k) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
-  if (x->dtype == TTN_F64) tt_merge_diag(x->r, k); else tt_merge_diag(x->c, k);
+  write_ttv(x).visit([&](auto& t) { tt_merge_diag(t, k); });
   API_END
 }
 int ttn_split_site(ttn_ttv x, int k, int64_t coarse, int mode, int64_t max_bond, double tol) {
   API_BEGIN
   need_init();
-  ttn_assert(x != nullptr, TTN_EARG, "null handle");
   ttn_assert(mode == 0 || mode == 1, TTN_EARG, "mode must be 0 (relative threshold) or 1 (tail norm)");
-  if (x->dtype == TTN_F64) tt_split_site(x->r, k, coarse, mode, max_bond, tol);
-  else tt_split_site(x->c, k, coarse, mode, max_bond, tol);
+  write_ttv(x).visit([&](auto& t) { tt_split_site(t, k, coarse, mode, max_bond, tol); });
   API_END
 }
 
@@ -638,118 +592,94 @@ int ttn_tdvp_params_default(ttn_tdvp_params* p) {
   return TTN_OK;
 }
 
-#define SOLVER_PROLOGUE(A, x0)                                         \
-  need_init();                                                         \
-  ttn_assert(A && x0 && p && x, TTN_EARG, "null argument");            \
-  same_dtype(A->dtype, x0->dtype);                                     \
-  ttn_ttv h = new ttn_ttv_s();                                         \
-  h->dtype = x0->dtype;
+}  // extern "C"
+// The prologue of every solver wrapper: A, x0 and the result share x0's element type; run(T tag, A, x0, x) runs the sweep
+// into the new train, which is handed out once it has returned.
+template <class F>
+static void solve(ttn_tto A, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, F&& run) {
+  need_init();
+  ttn_assert(A && p && x, TTN_EARG, "null argument");
+  ttn_ttv_s& x0s = read_ttv(x0);
+  same_dtype(A->dtype, x0s.dtype);
+  auto h = new_ttv(x0s.dtype);
+  with_dtype(x0s.dtype, [&](auto t) { using T = decltype(t); run(t, A->as<T>(), x0s.as<T>(), h->as<T>()); });
+  *x = h.release();
+}
+// the right-hand side of a linear solve, of A's element type
+static ttn_ttv_s& rhs(ttn_tto A, ttn_ttv b) {
+  ttn_ttv_s& bs = read_ttv(b);
+  ttn_assert(A != nullptr, TTN_EARG, "null argument");
+  same_dtype(A->dtype, bs.dtype);
+  return bs;
+}
+// the eigenvalue (and rank) history of a sweep, as far as the caller's arrays reach
+static void history_out(const std::vector<double>& Ev, const std::vector<int64_t>& rh, double* E, int64_t* r_hist, int cap_E,
+                        int* n_E) {
+  if (n_E) *n_E = (int)Ev.size();
+  for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) {
+    if (E) E[i] = Ev[i];
+    if (r_hist) r_hist[i] = rh[i];
+  }
+}
+extern "C" {
 
 int ttn_als_linsolve(ttn_tto A, ttn_ttv b, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* residual) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    ttn_assert(b != nullptr, TTN_EARG, "null argument");
-    same_dtype(A->dtype, b->dtype);
-    if (x0->dtype == TTN_F64) als_linsolve(A->r, b->r, x0->r, *p, h->r, residual);
-    else als_linsolve(A->c, b->c, x0->c, *p, h->c, residual);
-  } catch (...) { delete h; throw; }
-  *x = h;
+  ttn_ttv_s& bs = rhs(A, b);
+  solve(A, x0, p, x, [&](auto t, auto& At, auto& x0t, auto& xt) { als_linsolve(At, bs.as<decltype(t)>(), x0t, *p, xt, residual); });
   API_END
 }
 int ttn_als_eigsolve(ttn_tto A, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* E, int cap_E, int* n_E) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    std::vector<double> Ev;
-    if (x0->dtype == TTN_F64) als_eigsolve(A->r, x0->r, *p, h->r, Ev);
-    else als_eigsolve(A->c, x0->c, *p, h->c, Ev);
-    if (n_E) *n_E = (int)Ev.size();
-    if (E) for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) E[i] = Ev[i];
-  } catch (...) { delete h; throw; }
-  *x = h;
+  std::vector<double> Ev;
+  solve(A, x0, p, x, [&](auto, auto& At, auto& x0t, auto& xt) { als_eigsolve(At, x0t, *p, xt, Ev); });
+  history_out(Ev, {}, E, nullptr, cap_E, n_E);
   API_END
 }
 int ttn_als_gen_eigsolv(ttn_tto A, ttn_tto S, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* E, int cap_E, int* n_E) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    ttn_assert(S != nullptr, TTN_EARG, "null argument");
-    same_dtype(A->dtype, S->dtype);
-    std::vector<double> Ev;
-    if (x0->dtype == TTN_F64) als_gen_eigsolve(A->r, S->r, x0->r, *p, h->r, Ev);
-    else als_gen_eigsolve(A->c, S->c, x0->c, *p, h->c, Ev);
-    if (n_E) *n_E = (int)Ev.size();
-    if (E) for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) E[i] = Ev[i];
-  } catch (...) { delete h; throw; }
-  *x = h;
+  ttn_assert(A && S, TTN_EARG, "null argument");
+  same_dtype(A->dtype, S->dtype);
+  std::vector<double> Ev;
+  solve(A, x0, p, x, [&](auto t, auto& At, auto& x0t, auto& xt) { als_gen_eigsolve(At, S->as<decltype(t)>(), x0t, *p, xt, Ev); });
+  history_out(Ev, {}, E, nullptr, cap_E, n_E);
   API_END
 }
 int ttn_mals_linsolve(ttn_tto A, ttn_ttv b, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* residual) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    ttn_assert(b != nullptr, TTN_EARG, "null argument");
-    same_dtype(A->dtype, b->dtype);
-    if (x0->dtype == TTN_F64) mals_linsolve(A->r, b->r, x0->r, *p, h->r, residual);
-    else mals_linsolve(A->c, b->c, x0->c, *p, h->c, residual);
-  } catch (...) { delete h; throw; }
-  *x = h;
+  ttn_ttv_s& bs = rhs(A, b);
+  solve(A, x0, p, x, [&](auto t, auto& At, auto& x0t, auto& xt) { mals_linsolve(At, bs.as<decltype(t)>(), x0t, *p, xt, residual); });
   API_END
 }
 int ttn_mals_eigsolve(ttn_tto A, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* E, int64_t* r_hist, int cap_E,
                       int* n_E) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    std::vector<double> Ev;
-    std::vector<int64_t> rh;
-    if (x0->dtype == TTN_F64) mals_eigsolve(A->r, x0->r, *p, h->r, Ev, rh);
-    else mals_eigsolve(A->c, x0->c, *p, h->c, Ev, rh);
-    if (n_E) *n_E = (int)Ev.size();
-    for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) {
-      if (E) E[i] = Ev[i];
-      if (r_hist) r_hist[i] = rh[i];
-    }
-  } catch (...) { delete h; throw; }
-  *x = h;
+  std::vector<double> Ev;
+  std::vector<int64_t> rh;
+  solve(A, x0, p, x, [&](auto, auto& At, auto& x0t, auto& xt) { mals_eigsolve(At, x0t, *p, xt, Ev, rh); });
+  history_out(Ev, rh, E, r_hist, cap_E, n_E);
   API_END
 }
 int ttn_dmrg_linsolve(ttn_tto A, ttn_ttv b, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* residual) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    ttn_assert(b != nullptr, TTN_EARG, "null argument");
-    same_dtype(A->dtype, b->dtype);
-    if (x0->dtype == TTN_F64) dmrg_linsolve(A->r, b->r, x0->r, *p, h->r, residual);
-    else dmrg_linsolve(A->c, b->c, x0->c, *p, h->c, residual);
-  } catch (...) { delete h; throw; }
-  *x = h;
+  ttn_ttv_s& bs = rhs(A, b);
+  solve(A, x0, p, x, [&](auto t, auto& At, auto& x0t, auto& xt) { dmrg_linsolve(At, bs.as<decltype(t)>(), x0t, *p, xt, residual); });
   API_END
 }
 int ttn_dmrg_eigsolve(ttn_tto A, ttn_ttv x0, const ttn_solver_params* p, ttn_ttv* x, double* E, int64_t* r_hist, int cap_E,
                       int* n_E) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
-  try {
-    std::vector<double> Ev;
-    std::vector<int64_t> rh;
-    if (x0->dtype == TTN_F64) dmrg_eigsolve(A->r, x0->r, *p, h->r, Ev, rh);
-    else dmrg_eigsolve(A->c, x0->c, *p, h->c, Ev, rh);
-    if (n_E) *n_E = (int)Ev.size();
-    for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) {
-      if (E) E[i] = Ev[i];
-      if (r_hist) r_hist[i] = rh[i];
-    }
-  } catch (...) { delete h; throw; }
-  *x = h;
+  std::vector<double> Ev;
+  std::vector<int64_t> rh;
+  solve(A, x0, p, x, [&](auto, auto& At, auto& x0t, auto& xt) { dmrg_eigsolve(At, x0t, *p, xt, Ev, rh); });
+  history_out(Ev, rh, E, r_hist, cap_E, n_E);
   API_END
 }
 // ---- multi-GPU DMRG: replicated sweep, sharded Lanczos matvec (shard.cu) -----------------------------------------
 int ttn_shard_ctx_create(int dtype, int64_t max_elems, int rank, int nranks, ttn_shard_ctx* out) {
   API_BEGIN
   need_init();
-  ttn_assert(out != nullptr && (dtype == TTN_F64 || dtype == TTN_C128), TTN_EARG, "shard ctx: bad arguments");
+  ttn_assert(out != nullptr, TTN_EARG, "shard ctx: bad arguments");
   *out = shard_ctx_create(dtype, max_elems, rank, nranks);
   API_END
 }
@@ -767,42 +697,43 @@ int ttn_shard_ctx_bind(ttn_shard_ctx c, const void* all_handles) {
 }
 int ttn_shard_ctx_free(ttn_shard_ctx c) {
   API_BEGIN
-  if (c) shard_ctx_free(c);
+  delete c;
   API_END
 }
 int ttn_dmrg_eigsolve_sharded(ttn_tto A, ttn_ttv x0, const ttn_solver_params* p, ttn_shard_ctx sc, ttn_ttv* x, double* E,
                               int64_t* r_hist, int cap_E, int* n_E) {
   API_BEGIN
-  SOLVER_PROLOGUE(A, x0)
   ttn_assert(sc != nullptr, TTN_EARG, "null shard context");
-  active_shard_ctx() = sc;
-  try {
-    std::vector<double> Ev;
-    std::vector<int64_t> rh;
-    if (x0->dtype == TTN_F64) dmrg_eigsolve(A->r, x0->r, *p, h->r, Ev, rh);
-    else dmrg_eigsolve(A->c, x0->c, *p, h->c, Ev, rh);
-    active_shard_ctx() = nullptr;
+  std::vector<double> Ev;
+  std::vector<int64_t> rh;
+  solve(A, x0, p, x, [&](auto t, auto& At, auto& x0t, auto& xt) {
+    same_dtype(sc->dtype, A->dtype);
+    dmrg_eigsolve(At, x0t, *p, xt, Ev, rh, &sc->as<decltype(t)>());
     ttn_assert(shard_ctx_error(sc) == 0, TTN_ECUDA,
                "sharded DMRG: a peer did not publish its slice within the epoch timeout (TTN_SHARD_TIMEOUT_S); the result is invalid");
-    if (n_E) *n_E = (int)Ev.size();
-    for (int i = 0; i < (int)Ev.size() && i < cap_E; ++i) {
-      if (E) E[i] = Ev[i];
-      if (r_hist) r_hist[i] = rh[i];
-    }
-  } catch (...) { active_shard_ctx() = nullptr; delete h; throw; }
-  *x = h;
+  });
+  history_out(Ev, rh, E, r_hist, cap_E, n_E);
   API_END
 }
 int ttn_tdvp(ttn_tto H, ttn_ttv u0, const ttn_tdvp_params* p, ttn_ttv* u) {
   API_BEGIN
   need_init();
-  ttn_assert(H && u0 && p && u, TTN_EARG, "null argument");
-  same_dtype(H->dtype, u0->dtype);
-  ttn_ttv h = new ttn_ttv_s();
-  try {
-    tdvp_drive(H, u0, *p, h);
-  } catch (...) { delete h; throw; }
-  *u = h;
+  ttn_assert(H && p && u, TTN_EARG, "null argument");
+  ttn_ttv_s& u0s = read_ttv(u0);
+  same_dtype(H->dtype, u0s.dtype);
+  // real-time evolution of a real state runs on its complex promotion (tdvp.jl:167-172)
+  const bool promote = u0s.dtype != TTN_C128 && !p->imaginary_time;
+  auto h = new_ttv(promote ? TTN_C128 : u0s.dtype);
+  if (promote) {
+    TT<zc> uc;
+    TTO<zc> Hc;
+    tt_to_complex(u0s.as<double>(), uc);
+    tto_to_complex(H->as<double>(), Hc);
+    tdvp_run(Hc, uc, *p, h->as<zc>());
+  } else {
+    with_dtype(u0s.dtype, [&](auto t) { using T = decltype(t); tdvp_run(H->as<T>(), u0s.as<T>(), *p, h->as<T>()); });
+  }
+  *u = h.release();
   API_END
 }
 
@@ -822,7 +753,7 @@ int ttn_gemm(int dtype, int M, int N, int K, const void* A, int64_t sAm, int64_t
   g.alpha = alpha; g.beta = beta;
   // the batch is the outer dimension, which gemm() splits into launches of at most 65535 CTAs along grid.z
   g.batch1 = 1; g.batch2 = batch; g.bA2 = bA; g.bB2 = bB; g.bC2 = bC;
-  if (dtype == TTN_F64) gemm<double>(g); else gemm<zc>(g);
+  with_dtype(dtype, [&](auto t) { gemm<decltype(t)>(g); });
   API_END
 }
 
@@ -830,8 +761,7 @@ int ttn_matvec2_host(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, 
                      const void* V, void* Y, int symmetrize) {
   API_BEGIN
   need_init();
-  if (dtype == TTN_F64) matvec2_host<double>(w_l, w_r, chi_l, chi_r, nn, G, Amid, H, V, Y, symmetrize != 0);
-  else matvec2_host<zc>(w_l, w_r, chi_l, chi_r, nn, G, Amid, H, V, Y, symmetrize != 0);
+  with_dtype(dtype, [&](auto t) { matvec2_host<decltype(t)>(w_l, w_r, chi_l, chi_r, nn, G, Amid, H, V, Y, symmetrize != 0); });
   API_END
 }
 int ttn_matvec2_create(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, const void* G, const void* Amid,
@@ -850,7 +780,7 @@ int ttn_matvec2_apply(ttn_matvec mv, const void* V_dev, void* Y_dev) {
 }
 int ttn_matvec2_free(ttn_matvec mv) {
   API_BEGIN
-  matvec2_free(mv);
+  delete mv;
   API_END
 }
 int ttn_shard_range(int chi, int rank, int nranks, int* c0, int* cp) {
@@ -908,23 +838,21 @@ int ttn_shard_matvec_error(ttn_shard_matvec mv, int* err) {
 }
 int ttn_shard_matvec_free(ttn_shard_matvec mv) {
   API_BEGIN
-  shard_free(mv);
+  delete mv;
   API_END
 }
 int ttn_env_left_host(int dtype, int n, int w_l, int w_r, int r_l, int r_r, const void* G, const void* x, const void* A,
                       void* Gout) {
   API_BEGIN
   need_init();
-  if (dtype == TTN_F64) env_host<double>(true, n, w_l, w_r, r_l, r_r, G, x, A, Gout);
-  else env_host<zc>(true, n, w_l, w_r, r_l, r_r, G, x, A, Gout);
+  with_dtype(dtype, [&](auto t) { env_host<decltype(t)>(true, n, w_l, w_r, r_l, r_r, G, x, A, Gout); });
   API_END
 }
 int ttn_env_right_host(int dtype, int n, int w_l, int w_r, int r_l, int r_r, const void* H, const void* x, const void* A,
                        void* Hout) {
   API_BEGIN
   need_init();
-  if (dtype == TTN_F64) env_host<double>(false, n, w_l, w_r, r_l, r_r, H, x, A, Hout);
-  else env_host<zc>(false, n, w_l, w_r, r_l, r_r, H, x, A, Hout);
+  with_dtype(dtype, [&](auto t) { env_host<decltype(t)>(false, n, w_l, w_r, r_l, r_r, H, x, A, Hout); });
   API_END
 }
 
@@ -955,8 +883,7 @@ int ttn_svdtrunc_host(int dtype, int m, int n, const void* A, int64_t max_bond, 
   API_BEGIN
   need_init();
   ttn_assert(m >= 1 && n >= 1 && max_bond >= 1, TTN_EARG, "svdtrunc: bad shape");
-  if (dtype == TTN_F64) svdtrunc_host<double>(m, n, A, max_bond, truncerr, U, s, Vt, r_out);
-  else svdtrunc_host<zc>(m, n, A, max_bond, truncerr, U, s, Vt, r_out);
+  with_dtype(dtype, [&](auto t) { svdtrunc_host<decltype(t)>(m, n, A, max_bond, truncerr, U, s, Vt, r_out); });
   API_END
 }
 
@@ -980,7 +907,7 @@ int ttn_heig_host(int dtype, int n, int nev, int batch, const void* G, double* l
   API_BEGIN
   need_init();
   ttn_assert(n >= 1 && nev >= 1 && nev <= n && batch >= 1, TTN_EARG, "heig: bad shape");
-  if (dtype == TTN_F64) heig_host<double>(n, nev, batch, G, lam, U, flags); else heig_host<zc>(n, nev, batch, G, lam, U, flags);
+  with_dtype(dtype, [&](auto t) { heig_host<decltype(t)>(n, nev, batch, G, lam, U, flags); });
   API_END
 }
 }
@@ -1002,7 +929,7 @@ int ttn_qr_host(int dtype, int m, int n, const void* A, void* Q, void* R) {
   API_BEGIN
   need_init();
   ttn_assert(m >= 1 && n >= 1, TTN_EARG, "qr: bad shape");
-  if (dtype == TTN_F64) qr_host<double>(m, n, A, Q, R); else qr_host<zc>(m, n, A, Q, R);
+  with_dtype(dtype, [&](auto t) { qr_host<decltype(t)>(m, n, A, Q, R); });
   API_END
 }
 

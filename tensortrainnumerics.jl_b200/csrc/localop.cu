@@ -9,6 +9,7 @@
 // 4·w·n²·chi³ + 2·w²·n⁴·chi² flops for the two-site window); all three run on the DMMA GEMM of gemm.cu and the
 // intermediates T1/T2 stay in HBM/L2 between them.  The dense assemblies K_full of the reference
 // (als.jl:58-63, mals.jl:148-157, dmrg.jl:49-54) are never formed.
+#include <memory>
 #include "solvers.h"
 
 namespace ttn {
@@ -315,20 +316,18 @@ void env_host(bool left, int n, int w_l, int w_r, int r_l, int r_r, const void* 
 
 ttn_matvec matvec2_create(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, const void* G, const void* Amid,
                           const void* H) {
-  ttn_matvec mv = new ttn_matvec_s();
+  auto mv = std::make_unique<ttn_matvec_s>();
   mv->dtype = dtype;
-  try {
-    if (dtype == TTN_F64) setup_from_host<double>(mv->r, mv->L, mv->R, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, false);
-    else setup_from_host<zc>(mv->c, mv->L, mv->R, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, false);
-  } catch (...) { delete mv; throw; }
-  return mv;
+  mv->visit([&](auto& op) { setup_from_host(op, mv->L, mv->R, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, false); });
+  return mv.release();
 }
 void matvec2_apply(ttn_matvec mv, const void* V, void* Y) {
   ttn_assert(mv != nullptr, 2, "null matvec handle");
-  if (mv->dtype == TTN_F64) mv->r.apply((const double*)V, (double*)Y);
-  else mv->c.apply((const zc*)V, (zc*)Y);
+  with_dtype(mv->dtype, [&](auto t) {
+    using T = decltype(t);
+    mv->as<T>().apply((const T*)V, (T*)Y);
+  });
 }
-void matvec2_free(ttn_matvec mv) { delete mv; }
 
 #define INST(T)                                                                                                          \
   template struct LocalOp<T>;                                                                                            \

@@ -15,6 +15,7 @@
 // buffers are double-buffered by epoch parity so that a rank running one matvec ahead never overwrites a vector a
 // slower peer is still reading.  All Krylov vector algebra stays replicated (bit-identical on every rank), so no
 // scalar all-reduce is needed.
+#include <memory>
 #include "solvers.h"
 
 namespace ttn {
@@ -87,28 +88,6 @@ unsigned long long shard_timeout_ns() {
 }
 
 }  // namespace
-
-template <class T>
-struct ShardOp {
-  int chi_l = 1, chi_r = 1, w_l = 1, w_r = 1, nn = 1, rank = 0, nranks = 1, c0 = 0, cp = 1;
-  DevBuf L, Rs, Wq, T1, T2, err;
-  const void* Lp = nullptr;                // L2[a,(y,d)] used by the last GEMM: L.p, or the sweep's environment itself (no copy)
-  void* Ybuf[2] = {nullptr, nullptr};      // cudaMalloc (IPC-exportable), full (chi_l, nn, chi_r) vectors
-  unsigned* flags = nullptr;               // cudaMalloc, [2][nranks] epoch counters (one row per buffer parity is not needed)
-  void* Ypeer[2][8] = {};
-  unsigned* flag_peer_h[8] = {};
-  DevBuf flag_peer_d;
-  std::vector<void*> opened;
-  bool bound = false;
-  unsigned epoch = 0;
-  int64_t size() const { return (int64_t)chi_l * nn * chi_r; }
-  ~ShardOp() {
-    for (void* p : opened) cudaIpcCloseMemHandle(p);
-    if (Ybuf[0]) cudaFree(Ybuf[0]);
-    if (Ybuf[1]) cudaFree(Ybuf[1]);
-    if (flags) cudaFree(flags);
-  }
-};
 
 // contiguous slice [c0, c0 + cp) of `chi` owned by `rank` (first chi % nranks ranks get one extra element)
 void shard_range(int chi, int rank, int nranks, int* c0, int* cp) {
@@ -259,13 +238,6 @@ namespace ttn {
 // of the symmetrised pair 0.5 (K + K^T) of dmrg.jl:241.
 // ---------------------------------------------------------------------------------------------------------------------
 template <class T>
-struct ShardCtxT {
-  ShardOp<T> op[2];
-  int rank = 0, nranks = 1;
-  int64_t max_elems = 0;
-};
-
-template <class T>
 static void shard_ctx_alloc(ShardCtxT<T>& c, int64_t max_elems, int rank, int nranks) {
   ttn_assert(nranks >= 1 && nranks <= 8 && rank >= 0 && rank < nranks && max_elems >= 1, 2, "shard ctx: bad arguments");
   c.rank = rank; c.nranks = nranks; c.max_elems = max_elems;
@@ -328,49 +300,39 @@ static bool shard_rebind(ShardOp<T>& op, int64_t max_elems, const T* Lc, int chi
   return true;
 }
 
-}  // namespace ttn
-
-struct ttn_shard_matvec_s {
-  int dtype = 0;
-  ttn::ShardOp<double> r;
-  ttn::ShardOp<ttn::zc> c;
-};
-
-namespace ttn {
-
 ttn_shard_matvec shard_create(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, const void* G, const void* Amid,
                               const void* H, int rank, int nranks) {
-  ttn_shard_matvec mv = new ttn_shard_matvec_s();
+  auto mv = std::make_unique<ttn_shard_matvec_s>();
   mv->dtype = dtype;
-  try {
-    if (dtype == TTN_F64) shard_setup<double>(mv->r, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, rank, nranks);
-    else shard_setup<zc>(mv->c, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, rank, nranks);
-  } catch (...) { delete mv; throw; }
-  return mv;
+  mv->visit([&](auto& op) { shard_setup(op, w_l, w_r, chi_l, chi_r, nn, G, Amid, H, rank, nranks); });
+  return mv.release();
+}
+
+static void export_handles(void* const* yb, unsigned* fl, void* out) {
+  ShardHandles h;
+  TTN_CUDA(cudaIpcGetMemHandle(&h.y[0], yb[0]));
+  TTN_CUDA(cudaIpcGetMemHandle(&h.y[1], yb[1]));
+  TTN_CUDA(cudaIpcGetMemHandle(&h.flags, fl));
+  memcpy(out, &h, sizeof(h));
 }
 
 void shard_handles(ttn_shard_matvec mv, void* out192) {
   ttn_assert(mv != nullptr && out192 != nullptr, 2, "null argument");
   static_assert(sizeof(ShardHandles) == 192, "three 64-byte IPC handles");
-  ShardHandles h;
-  void* const* yb = mv->dtype == TTN_F64 ? mv->r.Ybuf : mv->c.Ybuf;
-  unsigned* fl = mv->dtype == TTN_F64 ? mv->r.flags : mv->c.flags;
-  TTN_CUDA(cudaIpcGetMemHandle(&h.y[0], yb[0]));
-  TTN_CUDA(cudaIpcGetMemHandle(&h.y[1], yb[1]));
-  TTN_CUDA(cudaIpcGetMemHandle(&h.flags, fl));
-  memcpy(out192, &h, sizeof(h));
+  mv->visit([&](auto& op) { export_handles(op.Ybuf, op.flags, out192); });
 }
 
 void shard_bind_handles(ttn_shard_matvec mv, const void* all) {
   ttn_assert(mv != nullptr && all != nullptr, 2, "null argument");
-  if (mv->dtype == TTN_F64) shard_bind<double>(mv->r, reinterpret_cast<const ShardHandles*>(all));
-  else shard_bind<zc>(mv->c, reinterpret_cast<const ShardHandles*>(all));
+  mv->visit([&](auto& op) { shard_bind(op, reinterpret_cast<const ShardHandles*>(all)); });
 }
 
 void* shard_apply_any(ttn_shard_matvec mv, const void* V) {
   ttn_assert(mv != nullptr && V != nullptr, 2, "null argument");
-  if (mv->dtype == TTN_F64) return shard_apply<double>(mv->r, (const double*)V);
-  return shard_apply<zc>(mv->c, (const zc*)V);
+  return with_dtype(mv->dtype, [&](auto t) -> void* {
+    using T = decltype(t);
+    return shard_apply<T>(mv->as<T>(), (const T*)V);
+  });
 }
 
 template <class T>
@@ -397,99 +359,68 @@ static double shard_eig_t(ShardOp<T>& op, T* x, int krylovdim, int maxiter, doub
 // replicated Lanczos recurrence on bit-identical vectors, only the matvec is distributed
 double shard_eigsolve(ttn_shard_matvec mv, void* x, int krylovdim, int maxiter, double tol, int* matvecs) {
   ttn_assert(mv != nullptr && x != nullptr, 2, "null argument");
-  if (mv->dtype == TTN_F64) return shard_eig_t<double>(mv->r, (double*)x, krylovdim, maxiter, tol, matvecs);
-  return shard_eig_t<zc>(mv->c, (zc*)x, krylovdim, maxiter, tol, matvecs);
+  return with_dtype(mv->dtype, [&](auto t) {
+    using T = decltype(t);
+    return shard_eig_t<T>(mv->as<T>(), (T*)x, krylovdim, maxiter, tol, matvecs);
+  });
 }
 
-int shard_error(ttn_shard_matvec mv) {
+static int read_err(const DevBuf& err) {
   int e = 0;
-  void* p = mv->dtype == TTN_F64 ? mv->r.err.p : mv->c.err.p;
-  read_back(&e, p, sizeof(int));
+  read_back(&e, err.p, sizeof(int));
   return e;
 }
 
-void shard_slice(ttn_shard_matvec mv, int* c0, int* cp) {
-  *c0 = mv->dtype == TTN_F64 ? mv->r.c0 : mv->c.c0;
-  *cp = mv->dtype == TTN_F64 ? mv->r.cp : mv->c.cp;
+int shard_error(ttn_shard_matvec mv) {
+  return mv->visit([](auto& op) { return read_err(op.err); });
 }
 
-void shard_free(ttn_shard_matvec mv) { delete mv; }
-
-}  // namespace ttn
-
-struct ttn_shard_ctx_s {
-  int dtype = 0;
-  ttn::ShardCtxT<double> r;
-  ttn::ShardCtxT<ttn::zc> c;
-};
-
-namespace ttn {
+void shard_slice(ttn_shard_matvec mv, int* c0, int* cp) {
+  mv->visit([&](auto& op) { *c0 = op.c0; *cp = op.cp; });
+}
 
 ttn_shard_ctx shard_ctx_create(int dtype, int64_t max_elems, int rank, int nranks) {
-  ttn_shard_ctx c = new ttn_shard_ctx_s();
+  auto c = std::make_unique<ttn_shard_ctx_s>();
   c->dtype = dtype;
-  try {
-    if (dtype == TTN_F64) shard_ctx_alloc<double>(c->r, max_elems, rank, nranks);
-    else shard_ctx_alloc<zc>(c->c, max_elems, rank, nranks);
-  } catch (...) { delete c; throw; }
-  return c;
+  c->visit([&](auto& sc) { shard_ctx_alloc(sc, max_elems, rank, nranks); });
+  return c.release();
 }
 // 2 x 192 bytes: the IPC handles of the two operators' exchange buffers
 void shard_ctx_handles(ttn_shard_ctx c, void* out384) {
   ttn_assert(c != nullptr && out384 != nullptr, 2, "null argument");
-  for (int t = 0; t < 2; ++t) {
-    ShardHandles h;
-    void* const* yb = c->dtype == TTN_F64 ? c->r.op[t].Ybuf : c->c.op[t].Ybuf;
-    unsigned* fl = c->dtype == TTN_F64 ? c->r.op[t].flags : c->c.op[t].flags;
-    TTN_CUDA(cudaIpcGetMemHandle(&h.y[0], yb[0]));
-    TTN_CUDA(cudaIpcGetMemHandle(&h.y[1], yb[1]));
-    TTN_CUDA(cudaIpcGetMemHandle(&h.flags, fl));
-    memcpy(reinterpret_cast<char*>(out384) + t * sizeof(ShardHandles), &h, sizeof(h));
-  }
+  c->visit([&](auto& sc) {
+    for (int t = 0; t < 2; ++t) export_handles(sc.op[t].Ybuf, sc.op[t].flags, reinterpret_cast<char*>(out384) + t * sizeof(ShardHandles));
+  });
 }
 void shard_ctx_bind(ttn_shard_ctx c, const void* all) {
   ttn_assert(c != nullptr && all != nullptr, 2, "null argument");
   const ShardHandles* hs = reinterpret_cast<const ShardHandles*>(all);
-  for (int t = 0; t < 2; ++t) {
-    if (c->dtype == TTN_F64) shard_bind<double>(c->r.op[t], hs + t, 2);
-    else shard_bind<zc>(c->c.op[t], hs + t, 2);
-  }
+  c->visit([&](auto& sc) { for (int t = 0; t < 2; ++t) shard_bind(sc.op[t], hs + t, 2); });
 }
-void shard_ctx_free(ttn_shard_ctx c) { delete c; }
 int shard_ctx_error(ttn_shard_ctx c) {
-  int e = 0, tot = 0;
-  for (int t = 0; t < 2; ++t) {
-    void* p = c->dtype == TTN_F64 ? c->r.op[t].err.p : c->c.op[t].err.p;
-    read_back(&e, p, sizeof(int));
-    tot |= e;
-  }
-  return tot;
+  return c->visit([](auto& sc) { return read_err(sc.op[0].err) | read_err(sc.op[1].err); });
 }
 
 // installs the sharded matvec on `lop` for the current window; false: the window is not sharded (too small), lop unchanged
 template <class T>
-bool shard_install(ttn_shard_ctx c, LocalOp<T>& lop, const T* Lc, const T* Rc, const T* Wf) {
-  if (c == nullptr) return false;
-  ShardCtxT<T>* sc = nullptr;
-  if (std::is_same<T, double>::value) { if (c->dtype != TTN_F64) return false; sc = reinterpret_cast<ShardCtxT<T>*>(&c->r); }
-  else { if (c->dtype != TTN_C128) return false; sc = reinterpret_cast<ShardCtxT<T>*>(&c->c); }
-  if (sc->nranks <= 1 || !sc->op[0].bound || lop.zero_site) return false;
-  if (!shard_rebind<T>(sc->op[0], sc->max_elems, Lc, lop.chi_l, lop.w_l, Rc, lop.chi_r, lop.w_r, Wf, lop.nn, false)) return false;
+bool shard_install(ShardCtxT<T>& sc, LocalOp<T>& lop, const T* Lc, const T* Rc, const T* Wf) {
+  if (sc.nranks <= 1 || !sc.op[0].bound || lop.zero_site) return false;
+  if (!shard_rebind<T>(sc.op[0], sc.max_elems, Lc, lop.chi_l, lop.w_l, Rc, lop.chi_r, lop.w_r, Wf, lop.nn, false)) return false;
   const bool sym = lop.symmetrize;
-  if (sym && !shard_rebind<T>(sc->op[1], sc->max_elems, Lc, lop.chi_l, lop.w_l, Rc, lop.chi_r, lop.w_r, Wf, lop.nn, true)) return false;
+  if (sym && !shard_rebind<T>(sc.op[1], sc.max_elems, Lc, lop.chi_l, lop.w_l, Rc, lop.chi_r, lop.w_r, Wf, lop.nn, true)) return false;
   const int64_t nel = lop.size();
-  lop.ext_apply = [sc, sym, nel](const T* V, T* Y) {
-    const T* Y1 = shard_apply<T>(sc->op[0], V);
+  lop.ext_apply = [&sc, sym, nel](const T* V, T* Y) {
+    const T* Y1 = shard_apply<T>(sc.op[0], V);
     TTN_CUDA(cudaMemcpyAsync(Y, Y1, sizeof(T) * (size_t)nel, cudaMemcpyDeviceToDevice, ctx().stream));
     if (sym) {
-      const T* Y2 = shard_apply<T>(sc->op[1], V);
+      const T* Y2 = shard_apply<T>(sc.op[1], V);
       axpy<T>(nel, t_one<T>(), Y2, Y);
       scal<T>(nel, t_from<T>(0.5, 0.0), Y);
     }
   };
   return true;
 }
-template bool shard_install<double>(ttn_shard_ctx, LocalOp<double>&, const double*, const double*, const double*);
-template bool shard_install<zc>(ttn_shard_ctx, LocalOp<zc>&, const zc*, const zc*, const zc*);
+template bool shard_install<double>(ShardCtxT<double>&, LocalOp<double>&, const double*, const double*, const double*);
+template bool shard_install<zc>(ShardCtxT<zc>&, LocalOp<zc>&, const zc*, const zc*, const zc*);
 
 }  // namespace ttn

@@ -92,10 +92,14 @@ void mals_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p,
                    std::vector<int64_t>& r_hist);
 template <class T>
 void dmrg_linsolve(const TTO<T>& A, const TT<T>& b, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, double* residual);
+template <class T> struct ShardCtxT;
+// shard: multi-GPU context whose ranks run the same sweep with the Lanczos matvec sharded over them (nullptr: one GPU)
 template <class T>
 void dmrg_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, std::vector<double>& E,
-                   std::vector<int64_t>& r_hist);
-void tdvp_drive(ttn_tto H, ttn_ttv u0, const ttn_tdvp_params& p, ttn_ttv out);
+                   std::vector<int64_t>& r_hist, ShardCtxT<T>* shard = nullptr);
+// tdvp.jl:45-357 on a state of the operator's element type (real-time evolution needs ComplexF64)
+template <class T>
+void tdvp_run(const TTO<T>& H, const TT<T>& u0, const ttn_tdvp_params& p, TT<T>& psi);
 
 // kernel-level test / benchmark entry points
 template <class T>
@@ -106,12 +110,44 @@ void env_host(bool left, int n, int w_l, int w_r, int r_l, int r_r, const void* 
 
 }  // namespace ttn
 
-struct ttn_matvec_s {
-  int dtype = 0;
-  ttn::LocalOp<double> r;
-  ttn::LocalOp<ttn::zc> c;
+struct ttn_matvec_s : ttn::ByDtype<ttn::LocalOp> {
   ttn::DevBuf L, R;
 };
+namespace ttn {
+// Effective-operator matvec sharded over the GPUs of one node (shard.cu): rank `rank` owns the bra slice [c0, c0 + cp) of
+// the right environment, and the last GEMM's epilogue stores every finished tile to all peers as well.
+template <class T>
+struct ShardOp {
+  int chi_l = 1, chi_r = 1, w_l = 1, w_r = 1, nn = 1, rank = 0, nranks = 1, c0 = 0, cp = 1;
+  DevBuf L, Rs, Wq, T1, T2, err;
+  const void* Lp = nullptr;                // L2[a,(y,d)] used by the last GEMM: L.p, or the sweep's environment itself (no copy)
+  void* Ybuf[2] = {nullptr, nullptr};      // cudaMalloc (IPC-exportable), full (chi_l, nn, chi_r) vectors
+  unsigned* flags = nullptr;               // cudaMalloc, [2][nranks] epoch counters (one row per buffer parity is not needed)
+  void* Ypeer[2][8] = {};
+  unsigned* flag_peer_h[8] = {};
+  DevBuf flag_peer_d;
+  std::vector<void*> opened;
+  bool bound = false;
+  unsigned epoch = 0;
+  int64_t size() const { return (int64_t)chi_l * nn * chi_r; }
+  ~ShardOp() {
+    for (void* p : opened) cudaIpcCloseMemHandle(p);
+    if (Ybuf[0]) cudaFree(Ybuf[0]);
+    if (Ybuf[1]) cudaFree(Ybuf[1]);
+    if (flags) cudaFree(flags);
+  }
+};
+// The sharded operator inside a DMRG sweep: exchange buffers allocated once per solve at the largest window size; op[1] is
+// the transposed operator of the symmetrised pair 0.5 (K + K^T) of dmrg.jl:241.
+template <class T>
+struct ShardCtxT {
+  ShardOp<T> op[2];
+  int rank = 0, nranks = 1;
+  int64_t max_elems = 0;
+};
+}  // namespace ttn
+struct ttn_shard_matvec_s : ttn::ByDtype<ttn::ShardOp> {};
+struct ttn_shard_ctx_s : ttn::ByDtype<ttn::ShardCtxT> {};
 typedef struct ttn_shard_matvec_s* ttn_shard_matvec;
 typedef struct ttn_shard_ctx_s* ttn_shard_ctx;
 namespace ttn {
@@ -119,10 +155,9 @@ namespace ttn {
 ttn_shard_ctx shard_ctx_create(int dtype, int64_t max_elems, int rank, int nranks);
 void shard_ctx_handles(ttn_shard_ctx c, void* out384);
 void shard_ctx_bind(ttn_shard_ctx c, const void* all);
-void shard_ctx_free(ttn_shard_ctx c);
 int shard_ctx_error(ttn_shard_ctx c);
-template <class T> bool shard_install(ttn_shard_ctx c, LocalOp<T>& lop, const T* Lc, const T* Rc, const T* Wf);
-ttn_shard_ctx& active_shard_ctx();   // per host thread; set by ttn_dmrg_eigsolve_sharded around the sweep
+// installs the sharded matvec on `lop` for the current window; false: the window is not sharded (too small), lop unchanged
+template <class T> bool shard_install(ShardCtxT<T>& sc, LocalOp<T>& lop, const T* Lc, const T* Rc, const T* Wf);
 // sharded effective operator (shard.cu)
 void shard_range(int chi, int rank, int nranks, int* c0, int* cp);
 ttn_shard_matvec shard_create(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, const void* G, const void* Amid,
@@ -133,9 +168,7 @@ void* shard_apply_any(ttn_shard_matvec mv, const void* V);
 double shard_eigsolve(ttn_shard_matvec mv, void* x, int krylovdim, int maxiter, double tol, int* matvecs);
 int shard_error(ttn_shard_matvec mv);
 void shard_slice(ttn_shard_matvec mv, int* c0, int* cp);
-void shard_free(ttn_shard_matvec mv);
 ttn_matvec matvec2_create(int dtype, int w_l, int w_r, int chi_l, int chi_r, int nn, const void* G, const void* Amid,
                           const void* H);
 void matvec2_apply(ttn_matvec mv, const void* V, void* Y);
-void matvec2_free(ttn_matvec mv);
 }  // namespace ttn

@@ -623,11 +623,6 @@ void mals_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p,
   }
 }
 
-ttn_shard_ctx& active_shard_ctx() {
-  static thread_local ttn_shard_ctx c = nullptr;
-  return c;
-}
-
 // ---------------------------------------------------------------------------------------------------------
 // DMRG (src/solvers/dmrg.jl:385-473, :501-578), N in {1, 2}
 // ---------------------------------------------------------------------------------------------------------
@@ -635,14 +630,15 @@ template <class T>
 struct DmrgLocal {
   const ttn_solver_params& p;
   bool lin;
-  DmrgLocal(const ttn_solver_params& p_, bool lin_) : p(p_), lin(lin_) {}
+  ShardCtxT<T>* shard;
+  DmrgLocal(const ttn_solver_params& p_, bool lin_, ShardCtxT<T>* shard_) : p(p_), lin(lin_), shard(shard_) {}
   // solves the local problem at window k in place on V (holding the initial guess); returns lambda for eig
   double solve(Sweeper<T>& S, int k, int N, DevBuf& V) {
     LocalOp<T> op; DevBuf W;
     S.setup_op(op, W, k, N, p.symmetrize != 0);
     // multi-GPU: the matvec of this window sharded over the ranks (shard.cu); windows too small to shard stay local
-    if (!lin && active_shard_ctx() != nullptr)
-      shard_install<T>(active_shard_ctx(), op, S.L[k].template as<T>(), S.R[k + N].template as<T>(), W.as<T>());
+    if (!lin && shard != nullptr)
+      shard_install<T>(*shard, op, S.L[k].template as<T>(), S.R[k + N].template as<T>(), W.as<T>());
     const int kd = std::max(p.krylovdim, 2), maxit = std::max(p.linsolv_maxiter, 1);
     if (lin) {
       DevBuf Pb;
@@ -726,7 +722,7 @@ static void dmrg_final_split(Sweeper<T>& S, int N, DevBuf& V, double tol, int64_
 
 template <class T>
 static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x,
-                     std::vector<double>* E, std::vector<int64_t>* r_hist, double* residual) {
+                     std::vector<double>* E, std::vector<int64_t>* r_hist, double* residual, ShardCtxT<T>* shard) {
   check_schedules(p);
   const int N = p.N;
   ttn_assert(N == 1 || N == 2, 2, "dmrg: window size N must be 1 or 2");
@@ -749,7 +745,7 @@ static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn
   if (E) E->clear();
   if (r_hist) r_hist->clear();
   S.init_right(N);
-  DmrgLocal<T> loc(p, lin);
+  DmrgLocal<T> loc(p, lin, shard);
   DevBuf V;
   S.window(0, N, V);   // V0 = b_mid(tt_opt, 1, N)   (dmrg.jl:275-276)
   auto maxrank = [&]() { int64_t m = 0; for (auto r : x.rks) m = std::max(m, r); return m; };
@@ -792,12 +788,12 @@ static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn
 
 template <class T>
 void dmrg_linsolve(const TTO<T>& A, const TT<T>& b, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, double* residual) {
-  dmrg_run<T>(A, &b, x0, p, x, nullptr, nullptr, residual);
+  dmrg_run<T>(A, &b, x0, p, x, nullptr, nullptr, residual, nullptr);
 }
 template <class T>
 void dmrg_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, std::vector<double>& E,
-                   std::vector<int64_t>& r_hist) {
-  dmrg_run<T>(A, nullptr, x0, p, x, &E, &r_hist, nullptr);
+                   std::vector<int64_t>& r_hist, ShardCtxT<T>* shard) {
+  dmrg_run<T>(A, nullptr, x0, p, x, &E, &r_hist, nullptr, shard);
 }
 
 #define INST(T)                                                                                                           \
@@ -811,7 +807,7 @@ void dmrg_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p,
                                  std::vector<int64_t>&);                                                                   \
   template void dmrg_linsolve<T>(const TTO<T>&, const TT<T>&, const TT<T>&, const ttn_solver_params&, TT<T>&, double*);    \
   template void dmrg_eigsolve<T>(const TTO<T>&, const TT<T>&, const ttn_solver_params&, TT<T>&, std::vector<double>&,      \
-                                 std::vector<int64_t>&);
+                                 std::vector<int64_t>&, ShardCtxT<T>*);
 INST(double)
 INST(zc)
 #undef INST

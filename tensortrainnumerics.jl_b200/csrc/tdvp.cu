@@ -235,6 +235,8 @@ struct Tdvp {
   }
 };
 
+}  // namespace
+
 template <class T>
 void tdvp_run(const TTO<T>& H, const TT<T>& u0, const ttn_tdvp_params& p, TT<T>& psi) {
   ttn_assert(p.n_steps >= 0 && (p.n_steps == 0 || p.steps), 2, "tdvp: bad steps");
@@ -263,23 +265,7 @@ void tdvp_run(const TTO<T>& H, const TT<T>& u0, const ttn_tdvp_params& p, TT<T>&
   }
 }
 
-}  // namespace
-
-void tdvp_drive(ttn_tto H, ttn_ttv u0, const ttn_tdvp_params& p, ttn_ttv out) {
-  const bool want_complex = !p.imaginary_time;   // tdvp.jl:167-172
-  if (u0->dtype == TTN_C128) {
-    out->dtype = TTN_C128;
-    tdvp_run<zc>(H->c, u0->c, p, out->c);
-  } else if (want_complex) {
-    TT<zc> uc; TTO<zc> Hc;
-    tt_to_complex(u0->r, uc);
-    tto_to_complex(H->r, Hc);
-    out->dtype = TTN_C128;
-    tdvp_run<zc>(Hc, uc, p, out->c);
-  } else {
-    out->dtype = TTN_F64;
-    tdvp_run<double>(H->r, u0->r, p, out->r);
-  }
-}
+template void tdvp_run<double>(const TTO<double>&, const TT<double>&, const ttn_tdvp_params&, TT<double>&);
+template void tdvp_run<zc>(const TTO<zc>&, const TT<zc>&, const ttn_tdvp_params&, TT<zc>&);
 
 }  // namespace ttn

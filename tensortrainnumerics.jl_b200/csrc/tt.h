@@ -1,6 +1,8 @@
 // Device-resident TT containers and the TT-level operations built from the kernels (internal).
 #pragma once
 #include "ttn_internal.h"
+#include "../../include/ttn_b200.h"
+#include <type_traits>
 
 namespace ttn {
 
@@ -84,14 +86,35 @@ int split_left(const T* Theta, int p, int q, int64_t rs, int64_t cs, bool conj, 
 
 }  // namespace ttn
 
+namespace ttn {
+// The element type behind a C-ABI dtype code: f(double{}) for TTN_F64, f(zc{}) for TTN_C128; any other code is TTN_EARG.
+template <class F>
+decltype(auto) with_dtype(int code, F&& f) {
+  if (code == TTN_F64) return f(double{});
+  ttn_assert(code == TTN_C128, TTN_EARG, "unknown dtype code");
+  return f(zc{});
+}
+
+// The Float64 and ComplexF64 instances of X behind one handle; `dtype` says which one is live.
+template <template <class> class X>
+struct ByDtype {
+  int dtype = TTN_F64;
+  X<double> r;
+  X<zc> c;
+  template <class T> X<T>& as() {
+    if constexpr (std::is_same<T, double>::value) return r; else return c;
+  }
+  template <class T> const X<T>& as() const { return const_cast<ByDtype*>(this)->template as<T>(); }
+  // f(as<T>()) for the live instance
+  template <class F> decltype(auto) visit(F&& f) { return with_dtype(dtype, [&](auto t) -> decltype(auto) { return f(as<decltype(t)>()); }); }
+};
+}  // namespace ttn
+
 // opaque handle types of the C ABI
-struct ttn_ttv_s {
-  int dtype = 0;
-  ttn::TT<double> r;
-  ttn::TT<ttn::zc> c;
+struct ttn_ttv_s : ttn::ByDtype<ttn::TT> {
   // asynchronous host <-> device traffic on the library's copy stream (ttn_ttv_upload_async / ttn_ttv_download_async):
-  cudaEvent_t ready = nullptr;   // recorded after the H2D copies: the compute stream must wait for it before the first use
-  cudaEvent_t busy = nullptr;    // recorded after the D2H copies: the cores must not be released before it
+  cudaEvent_t ready = nullptr;   // recorded after the H2D copies: the compute stream waits for it before the first use
+  cudaEvent_t busy = nullptr;    // recorded after the D2H copies: the cores must not be replaced or released before it
   // A handle freed while its D2H copies are still in flight parks its cores on the calling thread's deferred list (api.cu) and
   // they go back to the block cache once the event has completed, so the compute stream never waits for the copy engine.
   ~ttn_ttv_s();
@@ -100,8 +123,4 @@ namespace ttn {
 /// returns the cores of freed handles whose asynchronous downloads have completed to the block cache (`block`: wait for all)
 void drain_deferred_releases(bool block);
 }
-struct ttn_tto_s {
-  int dtype = 0;
-  ttn::TTO<double> r;
-  ttn::TTO<ttn::zc> c;
-};
+struct ttn_tto_s : ttn::ByDtype<ttn::TTO> {};
