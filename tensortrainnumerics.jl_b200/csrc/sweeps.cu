@@ -1,6 +1,6 @@
-// ALS / MALS / DMRG sweep drivers on device-resident trains.
+// ALS / MALS / DMRG / TDVP sweep drivers on device-resident trains.
 //
-// One engine serves the three solver families of the reference: the train `x`, canonical-layout left/right
+// One engine serves the four solver families of the reference: the train `x`, canonical-layout left/right
 // environments per bond (LocalOp docs in solvers.h), optional right-hand-side environments, and matrix-free
 // local solves.  The reference's pre-contracted environments (ALS `G` already multiplied by A_i,
 // als.jl:47-50; MALS 5-index `H` containing A_{i+1}, mals.jl:10-13) describe the same local operator
@@ -108,6 +108,31 @@ static void increase_ranks(TT<T>& x, int64_t max_bond) {
   x.rks = tgt;
   x.ot.assign(d, 0);
 }
+
+template <class T>
+static void orthogonalize_in_place(TT<T>& x) {  // tt_orthogonalize(x, 1) written back into x
+  TT<T> y;
+  tt_orthogonalize(x, 1, y);
+  x.cores = std::move(y.cores); x.rks = y.rks; x.ot = y.ot;
+}
+
+// The reference's sweep schedule: stage i ends when the sweep count reaches sweep_schedule[i] and the next stage starts with
+// that sweep; the solve ends with the last stage.
+struct SweepSchedule {
+  const ttn_solver_params& p;
+  int nsweeps = 0, stage = 0;
+  bool new_stage = false;  // the sweep started by the last next() opened a stage
+  explicit SweepSchedule(const ttn_solver_params& p_) : p(p_) {
+    ttn_assert(p.n_sweep_schedule >= 1 && p.n_sweep_schedule == p.n_rmax_schedule && p.sweep_schedule && p.rmax_schedule, 4,
+               "Sweep schedule error");
+  }
+  bool next() {  // starts a sweep; false once the last stage has ended
+    new_stage = (++nsweeps == p.sweep_schedule[stage]);
+    if (new_stage) ++stage;
+    return stage < p.n_sweep_schedule;
+  }
+  int64_t rmax() const { return p.rmax_schedule[stage]; }
+};
 
 // ---------------------------------------------------------------------------------------------------------
 // sweep state
@@ -274,18 +299,32 @@ struct Sweeper {
 };
 
 // ---------------------------------------------------------------------------------------------------------
+// QR right move shared by ALS (als.jl:104-136) and TDVP (tdvp.jl:83): the window V of site k, viewed as (chi_l n_k) x chi_r,
+// is factored V = Q R with r = min(chi_l n_k, chi_r); core k <- Q, bond k+1 <- r, R (r x chi_r) returned for the caller to absorb.
+// ---------------------------------------------------------------------------------------------------------
+template <class T>
+static int qr_right_move(Sweeper<T>& S, int k, DevBuf& V, DevBuf& R) {
+  const int cl = S.chi(k), cr = S.chi(k + 1), m = cl * S.n(k), r = std::min(m, cr);
+  DevBuf tau(sizeof(T) * (size_t)r), Q(sizeof(T) * (size_t)m * r);
+  R.alloc(sizeof(T) * (size_t)r * cr);
+  qr_factor<T>(V.as<T>(), m, cr, m, tau.as<T>());
+  qr_form_q<T>(V.as<T>(), m, r, m, tau.as<T>(), Q.as<T>(), m);
+  Copy4 t; t.n0 = r; t.n1 = cr; t.s0 = 1; t.s1 = m; t.d0 = 1; t.d1 = r; t.tri = 1;
+  copy4<T>(V.as<T>(), R.as<T>(), t);
+  S.store_core_from_rows(k, Q.as<T>(), cl, r);
+  S.x.rks[k + 1] = r;
+  return r;
+}
+
+// ---------------------------------------------------------------------------------------------------------
 // ALS core moves (src/solvers/als.jl:104-136): QR of the local solution, R absorbed into the neighbour
 // ---------------------------------------------------------------------------------------------------------
 template <class T>
 static void als_right_move(Sweeper<T>& S, int k, DevBuf& V) {
-  const int cl = S.chi(k), cr = S.chi(k + 1), nk = S.n(k), m = cl * nk;
-  ttn_assert(m >= cr, 1, "ALS: TT ranks exceed the local unfolding (over-full ranks)");
-  DevBuf tau(sizeof(T) * (size_t)cr), Q(sizeof(T) * (size_t)m * cr), Rb(sizeof(T) * (size_t)cr * cr);
-  qr_factor<T>(V.as<T>(), m, cr, m, tau.as<T>());
-  qr_form_q<T>(V.as<T>(), m, cr, m, tau.as<T>(), Q.as<T>(), m);
-  Copy4 t; t.n0 = cr; t.n1 = cr; t.s0 = 1; t.s1 = m; t.d0 = 1; t.d1 = cr; t.tri = 1;
-  copy4<T>(V.as<T>(), Rb.as<T>(), t);
-  S.store_core_from_rows(k, Q.as<T>(), cl, cr);
+  const int cr = S.chi(k + 1);
+  ttn_assert(S.chi(k) * S.n(k) >= cr, 1, "ALS: TT ranks exceed the local unfolding (over-full ranks)");
+  DevBuf Rb;
+  qr_right_move(S, k, V, Rb);
   S.x.ot[k] = -1;
   // x_{k+1}[s,kappa,c'] = sum_z R[kappa,z] x_{k+1}[s,z,c']
   const int n2 = S.n(k + 1), c2 = S.chi(k + 2);
@@ -338,7 +377,7 @@ static void als_left_move(Sweeper<T>& S, int k, DevBuf& V) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// SVD core moves shared by MALS (mals.jl:94-146) and DMRG (dmrg.jl:187-232).
+// SVD core moves shared by MALS (mals.jl:94-146), DMRG (dmrg.jl:187-232) and TDVP2 (tdvp.jl:250,278).
 // Theta = V viewed as (chi_l n_k) x (rest).  `rule` maps the sorted singular values to the retained rank.
 // right move: core k <- U, returns S·Vt (r x q);   left move: core `site` <- Vt, returns U·S (p x r)
 // ---------------------------------------------------------------------------------------------------------
@@ -408,14 +447,16 @@ void als_linsolve(const TTO<T>& A, const TT<T>& b, const TT<T>& x0, const ttn_so
 // ---------------------------------------------------------------------------------------------------------
 // als_eigsolve (src/solvers/als.jl:251-321), noise_schedule = 0
 // ---------------------------------------------------------------------------------------------------------
-static void check_schedules(const ttn_solver_params& p) {
-  ttn_assert(p.n_sweep_schedule >= 1 && p.n_sweep_schedule == p.n_rmax_schedule && p.sweep_schedule && p.rmax_schedule, 4,
-             "Sweep schedule error");
+// stage change: ranks raised to the stage's rmax by zero padding, then the train is left-orthogonalised again
+template <class T>
+static void als_next_stage(TT<T>& x, int64_t rmax) {
+  increase_ranks(x, rmax);
+  orthogonalize_in_place(x);
 }
 
 template <class T>
 void als_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, std::vector<double>& E) {
-  check_schedules(p);
+  SweepSchedule sched(p);
   tt_orthogonalize(x0, 1, x);
   E.clear();
   const int kd = std::max(p.krylovdim, 2), maxit = std::max(p.linsolv_maxiter, 1);
@@ -428,16 +469,9 @@ void als_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, 
     S->window(k, 1, V);
     return lanczos_lowest<T>(op, V.as<T>(), kd, maxit, p.linsolv_tol, nullptr);
   };
-  int nsweeps = 0, i_sched = 1;
-  while (i_sched <= p.n_sweep_schedule) {
-    ++nsweeps;
-    if (nsweeps == p.sweep_schedule[i_sched - 1]) {
-      ++i_sched;
-      if (i_sched > p.n_sweep_schedule) return;
-      increase_ranks(x, p.rmax_schedule[i_sched - 1]);
-      TT<T> y;
-      tt_orthogonalize(x, 1, y);
-      x.cores = std::move(y.cores); x.rks = y.rks; x.ot = y.ot;
+  while (sched.next()) {
+    if (sched.new_stage) {
+      als_next_stage(x, sched.rmax());
       S.reset(new Sweeper<T>(A, nullptr, x));
       S->init_right(1);
     }
@@ -463,7 +497,7 @@ void als_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, 
 template <class T>
 void als_gen_eigsolve(const TTO<T>& A, const TTO<T>& Sop, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x,
                       std::vector<double>& E) {
-  check_schedules(p);
+  SweepSchedule sched(p);
   tt_orthogonalize(x0, 1, x);
   E.clear();
   const int kd = std::max(p.krylovdim, 2), maxit = std::max(p.linsolv_maxiter, 1);
@@ -487,16 +521,9 @@ void als_gen_eigsolve(const TTO<T>& A, const TTO<T>& Sop, const TT<T>& x0, const
     }
     return lam;
   };
-  int nsweeps = 0, i_sched = 1;
-  while (i_sched <= p.n_sweep_schedule) {
-    ++nsweeps;
-    if (nsweeps == p.sweep_schedule[i_sched - 1]) {
-      ++i_sched;
-      if (i_sched > p.n_sweep_schedule) return;
-      increase_ranks(x, p.rmax_schedule[i_sched - 1]);
-      TT<T> y;
-      tt_orthogonalize(x, 1, y);
-      x.cores = std::move(y.cores); x.rks = y.rks; x.ot = y.ot;
+  while (sched.next()) {
+    if (sched.new_stage) {
+      als_next_stage(x, sched.rmax());
       SA.reset(new Sweeper<T>(A, nullptr, x));
       SS.reset(new Sweeper<T>(Sop, nullptr, x));
       SA->init_right(1);
@@ -583,7 +610,7 @@ void mals_linsolve(const TTO<T>& A, const TT<T>& b, const TT<T>& x0, const ttn_s
 template <class T>
 void mals_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, std::vector<double>& E,
                    std::vector<int64_t>& r_hist) {
-  check_schedules(p);
+  SweepSchedule sched(p);
   tt_orthogonalize(x0, 1, x);
   Sweeper<T> S(A, nullptr, x);
   const int d = S.d;
@@ -598,14 +625,8 @@ void mals_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p,
     return lanczos_lowest<T>(op, V.as<T>(), kd, maxit, p.linsolv_tol, nullptr);
   };
   auto maxrank = [&]() { int64_t m = 0; for (auto r : x.rks) m = std::max(m, r); return m; };
-  int nsweeps = 0, i_sched = 1;
-  while (i_sched <= p.n_sweep_schedule) {
-    ++nsweeps;
-    if (nsweeps == p.sweep_schedule[i_sched - 1]) {
-      ++i_sched;
-      if (i_sched > p.n_sweep_schedule) return;
-    }
-    const int64_t rmax = p.rmax_schedule[i_sched - 1];
+  while (sched.next()) {
+    const int64_t rmax = sched.rmax();
     for (int k = 0; k < d - 1; ++k) {
       DevBuf V;
       E.push_back(eig_win(k, V));
@@ -631,7 +652,9 @@ struct DmrgLocal {
   const ttn_solver_params& p;
   bool lin;
   ShardCtxT<T>* shard;
-  DmrgLocal(const ttn_solver_params& p_, bool lin_, ShardCtxT<T>* shard_) : p(p_), lin(lin_), shard(shard_) {}
+  int kd, maxit;
+  DmrgLocal(const ttn_solver_params& p_, bool lin_, ShardCtxT<T>* shard_)
+      : p(p_), lin(lin_), shard(shard_), kd(std::max(p.krylovdim, 2)), maxit(std::max(p.linsolv_maxiter, 1)) {}
   // solves the local problem at window k in place on V (holding the initial guess); returns lambda for eig
   double solve(Sweeper<T>& S, int k, int N, DevBuf& V) {
     LocalOp<T> op; DevBuf W;
@@ -639,7 +662,6 @@ struct DmrgLocal {
     // multi-GPU: the matvec of this window sharded over the ranks (shard.cu); windows too small to shard stay local
     if (!lin && shard != nullptr)
       shard_install<T>(*shard, op, S.L[k].template as<T>(), S.R[k + N].template as<T>(), W.as<T>());
-    const int kd = std::max(p.krylovdim, 2), maxit = std::max(p.linsolv_maxiter, 1);
     if (lin) {
       DevBuf Pb;
       S.local_rhs(k, N, Pb);
@@ -723,7 +745,7 @@ static void dmrg_final_split(Sweeper<T>& S, int N, DevBuf& V, double tol, int64_
 template <class T>
 static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x,
                      std::vector<double>* E, std::vector<int64_t>* r_hist, double* residual, ShardCtxT<T>* shard) {
-  check_schedules(p);
+  SweepSchedule sched(p);
   const int N = p.N;
   ttn_assert(N == 1 || N == 2, 2, "dmrg: window size N must be 1 or 2");
   const bool lin = (b != nullptr);
@@ -749,21 +771,8 @@ static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn
   DevBuf V;
   S.window(0, N, V);   // V0 = b_mid(tt_opt, 1, N)   (dmrg.jl:275-276)
   auto maxrank = [&]() { int64_t m = 0; for (auto r : x.rks) m = std::max(m, r); return m; };
-  int nsweeps = 0, i_sched = 1;
-  while (i_sched <= p.n_sweep_schedule) {
-    ++nsweeps;
-    if (nsweeps == p.sweep_schedule[i_sched - 1]) {
-      ++i_sched;
-      if (i_sched > p.n_sweep_schedule) {
-        const double lam = loc.solve(S, 0, N, V);
-        if (E) E->push_back(lam);
-        if (r_hist) r_hist->push_back(maxrank());
-        dmrg_final_split(S, N, V, p.tol, p.rmax_schedule[p.n_rmax_schedule - 1]);
-        if (residual) *residual = S.residual();
-        return;
-      }
-    }
-    const int64_t rmax = p.rmax_schedule[i_sched - 1];
+  while (sched.next()) {
+    const int64_t rmax = sched.rmax();
     for (int k = 0; k <= d - N - 1; ++k) {
       const double lam = loc.solve(S, k, N, V);
       if (E) E->push_back(lam);
@@ -783,7 +792,11 @@ static void dmrg_run(const TTO<T>& A, const TT<T>* b, const TT<T>& x0, const ttn
       if (r_hist) r_hist->push_back(maxrank());
     }
   }
-  if (residual && lin) *residual = S.residual();
+  const double lam = loc.solve(S, 0, N, V);
+  if (E) E->push_back(lam);
+  if (r_hist) r_hist->push_back(maxrank());
+  dmrg_final_split(S, N, V, p.tol, p.rmax_schedule[p.n_rmax_schedule - 1]);
+  if (residual) *residual = S.residual();
 }
 
 template <class T>
@@ -794,6 +807,174 @@ template <class T>
 void dmrg_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p, TT<T>& x, std::vector<double>& E,
                    std::vector<int64_t>& r_hist, ShardCtxT<T>* shard) {
   dmrg_run<T>(A, nullptr, x0, p, x, &E, &r_hist, nullptr, shard);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// TDVP / TDVP2 (src/solvers/tdvp.jl:45-357).  The one-, two- and zero-site effective operators of tdvp.jl:29-35,205-208 are
+// LocalOps of this engine (the (l,s,r) / (a,s_out,b,s_in) layouts of tdvp.jl:54-55 coincide with the window layout), the
+// environment recursions of tdvp.jl:37-43 are update_left / update_right, `exponentiate` is lanczos_expm, and the truncations
+// (tdvp.jl:250,278) are the SVD moves with the tail-norm rule.  A sweep carries the window AC of the orthogonality centre from
+// site 0 to the last site and back to site 0.
+// ---------------------------------------------------------------------------------------------------------
+// V <- exp(t K) V with t = (tre, tim) (KrylovKit.exponentiate, tdvp.jl:75); the Krylov settings are clamped once per solve
+struct Expm {
+  int kd, maxit;
+  double tol;
+  explicit Expm(const ttn_tdvp_params& p) : kd(std::max(p.krylovdim, 2)), maxit(std::max(p.krylov_maxiter, 1)), tol(p.krylov_tol) {}
+  template <class T>
+  void operator()(LocalOp<T>& op, DevBuf& V, double tre, double tim) const {
+    lanczos_expm<T>(op, V.as<T>(), tre, tim, kd, maxit, tol, nullptr);
+  }
+};
+// the same on the one- or two-site window at k
+template <class T>
+static void evolve(Sweeper<T>& S, const Expm& ex, int k, int N, DevBuf& V, double tre, double tim) {
+  LocalOp<T> op; DevBuf W;
+  S.setup_op(op, W, k, N, false);
+  ex(op, V, tre, tim);
+}
+
+// one-site sweep (tdvp.jl:45-152): each site forward by t1, each bond between two sites backward by t0
+template <class T>
+static void tdvp_sweep1(Sweeper<T>& S, const Expm& ex, DevBuf& AC, double t1re, double t1im, double t0re, double t0im) {
+  TT<T>& x = S.x;
+  const int d = S.d;
+  for (int k = 0; k < d - 1; ++k) {
+    evolve(S, ex, k, 1, AC, t1re, t1im);
+    const int cr = S.chi(k + 1);
+    DevBuf C;
+    const int r = qr_right_move(S, k, AC, C);
+    S.update_left(k);
+    {
+      LocalOp<T> op;   // bond k+1: L[k+1] has the new bond r, R[k+1] still the old bond cr; C is r x cr
+      op.setup(S.L[k + 1].template as<T>(), r, S.w(k + 1), S.R[k + 1].template as<T>(), cr, S.w(k + 1), nullptr, 1, false);
+      ex(op, C, t0re, t0im);
+    }
+    // AC[a,s,c] = sum_g C[a,g] x_{k+1}[s,g,c]
+    const int n2 = S.n(k + 1), c2 = S.chi(k + 2);
+    DevBuf ACn(sizeof(T) * (size_t)r * n2 * c2);
+    GemmArgs g;
+    g.M = r; g.N = c2; g.K = cr;
+    g.A = C.p; g.sAm = 1; g.sAk = r;
+    g.B = x.core(k + 1); g.sBk = n2; g.sBn = (int64_t)n2 * cr; g.bB1 = 1;
+    g.C = ACn.p; g.sCm = 1; g.sCn = (int64_t)r * n2; g.bC1 = r;
+    g.batch1 = n2;
+    gemm<T>(g);
+    AC = std::move(ACn);
+  }
+  evolve(S, ex, d - 1, 1, AC, t1re, t1im);
+  for (int k = d - 2; k >= 0; --k) {
+    // AC belongs to site k+1: (cl, n, cr);  LQ of cl x (n cr) via QR of the conjugate transpose.  Unlike als_left_move, which
+    // keeps R as factored and absorbs it transposed into the core on its left, the factor is taken as L = R^H: the bond
+    // matrix C that the zero-site step evolves.
+    const int cl = S.chi(k + 1), cr = S.chi(k + 2), nk = S.n(k + 1), m = nk * cr, r = std::min(cl, m);
+    DevBuf W(sizeof(T) * (size_t)m * cl), tau(sizeof(T) * (size_t)r), Q(sizeof(T) * (size_t)m * r), C(sizeof(T) * (size_t)cl * r);
+    Copy4 c;  // W[(s,c), a] = conj(AC[a,s,c])
+    c.n0 = m; c.s0 = cl; c.d0 = 1;
+    c.n1 = cl; c.s1 = 1; c.d1 = m;
+    c.conj = true;
+    copy4<T>(AC.as<T>(), W.as<T>(), c);
+    qr_factor<T>(W.as<T>(), m, cl, m, tau.as<T>());
+    qr_form_q<T>(W.as<T>(), m, r, m, tau.as<T>(), Q.as<T>(), m);
+    Copy4 t;  // C = L = R^H : C[a,kappa] = conj(R[kappa,a])
+    t.n0 = r; t.n1 = cl; t.s0 = 1; t.s1 = m; t.d0 = cl; t.d1 = 1; t.tri = 1; t.conj = true;
+    copy4<T>(W.as<T>(), C.as<T>(), t);
+    S.store_core_from_Vq(k + 1, Q.as<T>(), m, r, cr);   // x_{k+1}[s,kappa,c] = conj(Q[s + n c, kappa])
+    x.rks[k + 1] = r;
+    S.update_right(k + 1);
+    {
+      LocalOp<T> op;   // bond k+1: L[k+1] has the old bond cl, R[k+1] the new bond r; C is cl x r
+      op.setup(S.L[k + 1].template as<T>(), cl, S.w(k + 1), S.R[k + 1].template as<T>(), r, S.w(k + 1), nullptr, 1, false);
+      ex(op, C, t0re, t0im);
+    }
+    // AC[(a,s), g'] = sum_g x_k[(s,a), g] C[g,g']  -> window layout [a,s,g']
+    const int c0 = S.chi(k), n0 = S.n(k);
+    DevBuf ACn(sizeof(T) * (size_t)c0 * n0 * r);
+    GemmArgs g;
+    g.M = c0; g.N = r; g.K = cl;
+    g.A = x.core(k); g.sAm = n0; g.sAk = (int64_t)n0 * c0; g.bA1 = 1;
+    g.B = C.p; g.sBk = 1; g.sBn = cl; g.bB1 = 0;
+    g.C = ACn.p; g.sCm = 1; g.sCn = (int64_t)c0 * n0; g.bC1 = c0;
+    g.batch1 = n0;
+    gemm<T>(g);
+    AC = std::move(ACn);
+    evolve(S, ex, k, 1, AC, t1re, t1im);
+  }
+}
+
+// two-site sweep (tdvp.jl:210-301): each pair of sites forward by t2, each site between two pairs backward by t1
+template <class T, class Rule>
+static void tdvp_sweep2(Sweeper<T>& S, const Expm& ex, Rule rule, DevBuf& AC, double t2re, double t2im, double t1re,
+                        double t1im) {
+  const int d = S.d;
+  for (int k = 0; k < d - 1; ++k) {
+    const int cl = S.chi(k), cm = S.chi(k + 1), n1 = S.n(k), n2 = S.n(k + 1), cr = S.chi(k + 2);
+    DevBuf AAC(sizeof(T) * (size_t)cl * n1 * n2 * cr);
+    GemmArgs g;  // AAC[(a,s1),s2,c] = sum_g AC[(a,s1),g] x_{k+1}[s2,g,c]
+    g.M = cl * n1; g.N = cr; g.K = cm;
+    g.A = AC.p; g.sAm = 1; g.sAk = (int64_t)cl * n1;
+    g.B = S.x.core(k + 1); g.sBk = n2; g.sBn = (int64_t)n2 * cm; g.bB1 = 1;
+    g.C = AAC.p; g.sCm = 1; g.sCn = (int64_t)cl * n1 * n2; g.bC1 = (int64_t)cl * n1;
+    g.batch1 = n2;
+    gemm<T>(g);
+    evolve(S, ex, k, 2, AAC, t2re, t2im);
+    DevBuf SVt;
+    svd_right_move<T>(S, k, AAC.as<T>(), cl * n1, n2 * cr, rule, SVt);
+    S.update_left(k);
+    AC = std::move(SVt);   // (r, n2, cr) window of site k+1, whose core is not stored
+    if (k < d - 2) evolve(S, ex, k + 1, 1, AC, t1re, t1im);
+  }
+  for (int k = d - 2; k >= 0; --k) {
+    // AC is the window of site k+1: (cm, n2, cr)
+    const int cl = S.chi(k), cm = S.chi(k + 1), n1 = S.n(k), n2 = S.n(k + 1), cr = S.chi(k + 2);
+    DevBuf AAC(sizeof(T) * (size_t)cl * n1 * n2 * cr);
+    GemmArgs g;  // AAC[a,s1,(s2,c)] = sum_g x_k[s1,a,g] AC[g,(s2,c)]
+    g.M = cl; g.N = n2 * cr; g.K = cm;
+    g.A = S.x.core(k); g.sAm = n1; g.sAk = (int64_t)n1 * cl; g.bA1 = 1;
+    g.B = AC.p; g.sBk = 1; g.sBn = cm; g.bB1 = 0;
+    g.C = AAC.p; g.sCm = 1; g.sCn = (int64_t)cl * n1; g.bC1 = cl;
+    g.batch1 = n1;
+    gemm<T>(g);
+    evolve(S, ex, k, 2, AAC, t2re, t2im);
+    DevBuf US;
+    svd_left_move<T>(S, k + 1, AAC.as<T>(), cl * n1, n2 * cr, rule, US);
+    S.update_right(k + 1);
+    AC = std::move(US);   // (cl, n1, r) window of site k
+    if (k > 0) evolve(S, ex, k, 1, AC, t1re, t1im);
+  }
+}
+
+template <class T>
+void tdvp_run(const TTO<T>& H, const TT<T>& u0, const ttn_tdvp_params& p, TT<T>& psi) {
+  ttn_assert(p.n_steps >= 0 && (p.n_steps == 0 || p.steps), 2, "tdvp: bad steps");
+  ttn_assert(is_cplx<T>::value || p.imaginary_time, 2, "tdvp: real-time evolution needs a complex state");
+  const Expm ex(p);
+  auto rule = [&](const double* s, int len) { return rank_tailnorm(s, len, p.max_bond, p.truncerr); };
+  tt_orthogonalize(u0, 1, psi);
+  for (int is = 0; is < p.n_steps; ++is) {
+    const double h = p.steps[is];
+    // dt_eff = +i h (imaginary time) or h (real time);  t1 = -i dt_eff,  t0 = +i dt_eff   (tdvp.jl:74,94,179)
+    double t1re, t1im;
+    if (p.imaginary_time) { t1re = h; t1im = 0.0; } else { t1re = 0.0; t1im = -h; }
+    for (int s = 0; s < std::max(1, p.sweeps); ++s) {
+      Sweeper<T> S(H, nullptr, psi);
+      S.init_right(1);
+      DevBuf AC;
+      S.window(0, 1, AC);
+      if (p.two_site) tdvp_sweep2(S, ex, rule, AC, 0.5 * t1re, 0.5 * t1im, -0.5 * t1re, -0.5 * t1im);
+      else tdvp_sweep1(S, ex, AC, t1re, t1im, -t1re, -t1im);
+      S.store_core_from_rows(0, AC.as<T>(), S.chi(0), S.chi(1));
+      psi.ot.assign(psi.d, 0);
+    }
+    if (p.normalize) {
+      std::vector<T> nn;
+      tt_dot(psi, psi, nn);
+      const double nrm = std::sqrt(std::max(0.0, t_real(nn[0])));
+      ttn_assert(nrm > 0.0, 5, "tdvp: state norm vanished");
+      scal<T>(psi.core_elems(0), t_from<T>(1.0 / nrm, 0.0), psi.core(0));
+    }
+    orthogonalize_in_place(psi);
+  }
 }
 
 #define INST(T)                                                                                                           \
@@ -807,7 +988,8 @@ void dmrg_eigsolve(const TTO<T>& A, const TT<T>& x0, const ttn_solver_params& p,
                                  std::vector<int64_t>&);                                                                   \
   template void dmrg_linsolve<T>(const TTO<T>&, const TT<T>&, const TT<T>&, const ttn_solver_params&, TT<T>&, double*);    \
   template void dmrg_eigsolve<T>(const TTO<T>&, const TT<T>&, const ttn_solver_params&, TT<T>&, std::vector<double>&,      \
-                                 std::vector<int64_t>&, ShardCtxT<T>*);
+                                 std::vector<int64_t>&, ShardCtxT<T>*);                                                    \
+  template void tdvp_run<T>(const TTO<T>&, const TT<T>&, const ttn_tdvp_params&, TT<T>&);
 INST(double)
 INST(zc)
 #undef INST

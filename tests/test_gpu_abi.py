@@ -387,6 +387,30 @@ def test_tto_upload_rejects_empty_cores(zero):
     assert lib.ttn_tto_upload(F64, 2, dims, rks, cores, C.byref(out)) == EDIM
 
 
+@pytest.mark.parametrize("side", ["left", "right"])
+def test_tdvp_rejects_an_operator_with_boundary_rank_above_one(side):
+    """The boundary environments of a sweep are 1 x 1 x 1: ttn_tdvp refuses an operator whose first or last rank is 2 with
+    TTN_EDIM, like the other solvers, instead of reading that environment as 1 x 2 x 1."""
+    lib = _lib()
+    rng = np.random.default_rng(13)
+    dims, rks = [2, 2, 2], ([2, 2, 2, 1] if side == "left" else [1, 2, 2, 2])
+    host = [rng.standard_normal(n * n * rks[k] * rks[k + 1]) for k, n in enumerate(dims)]
+    i64 = lambda v: (C.c_int64 * len(v))(*v)  # noqa: E731
+    H = vp()
+    _check(lib.ttn_tto_upload(F64, 3, i64(dims), i64(rks), (vp * 3)(*[a.ctypes.data for a in host]), C.byref(H)))
+    x = Pinned((2,) * 3, [1, 2, 2, 1], np.float64, 1, rng).upload(asynchronous=False)
+    steps = (C.c_double * 1)(0.05)
+    p = _tdvp_params(steps)
+    p.imaginary_time = 1
+    out = vp()
+    try:
+        assert lib.ttn_tdvp(H, x, C.byref(p), C.byref(out)) == EDIM
+        assert not out.value
+    finally:
+        _check(lib.ttn_ttv_free(x))
+        _check(lib.ttn_tto_free(H))
+
+
 def test_sharded_dmrg_rejects_a_context_of_another_dtype():
     """A Float64 shard context with a ComplexF64 train and operator is TTN_EDIM, not a silent unsharded run."""
     lib = _lib()
